@@ -2,6 +2,7 @@
 """denovo3D candidates/sec (solve + score) on N B200s vs the reference CPU path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg2|cfg1|cfg3]
+                    [--dump-outputs DIR]
 
 Workload (default, BASELINE.json configs[1]): one synthetic amyloid-like filament image, 256x256 px at 1.3 A/px (true
 twist -1.2 deg, rise 4.75 A); dense 1000 twist x 50 rise grid; interpolation "nn", algorithm {"model": "lsq"}, cosine
@@ -332,6 +333,30 @@ def reference_arm(args, cfg, img, rank):
     return 0
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+NPY_HEADER_BYTES = 256  # np.save writes 128 B of header before a 1-D array; the limit counts whole files
+
+
+def dump_outputs(out_dir, per_candidate, top, limit=DUMP_LIMIT_BYTES, seed=2026):
+    """Write the results of the timed region as ``out_dir/<name>.npy`` so that two builds can be compared output for
+    output.  ``per_candidate`` maps names to arrays of equal length (one entry per slot of the score map);
+    ``candidate_index.npy`` gives the flat job index of each entry.  When these would exceed ``limit`` bytes, a fixed
+    seeded sample of the entries is written instead (``limit`` counts whole files, headers included).  ``top`` maps names
+    to the (short) top-K arrays."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v) for k, v in per_candidate.items()}
+    top = {k: np.asarray(v) for k, v in top.items()}
+    n = len(arrays["candidate_index"])
+    row_bytes = sum(a.dtype.itemsize for a in arrays.values())
+    room = limit - sum(a.nbytes for a in top.values()) - NPY_HEADER_BYTES * (len(arrays) + len(top))
+    if n * row_bytes > room:
+        keep = np.sort(np.random.default_rng(seed).choice(n, room // row_bytes, replace=False))
+        arrays = {k: a[keep] for k, a in arrays.items()}
+    for name, a in {**arrays, **top}.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def _ndisk(key):
     D2, L2, D3, D3i, s, L3 = key
     c = np.arange(D3) - D3 // 2
@@ -357,7 +382,14 @@ def main():
     ap.add_argument("--e2e-calls", type=int, default=3, help="timed search_grid() calls of the e2e measurement")
     ap.add_argument("--e2e-batches", type=int, default=2, help="batches per rank and search_grid() call of the e2e measurement")
     ap.add_argument("--ref-workers", type=int, default=0, help="--impl reference: worker processes (default: all cores)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the score map and top-K the timed steps computed as DIR/<name>.npy (float32/float64, "
+                         "<= 64 MB; a fixed seeded sample of a larger map)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -477,6 +509,11 @@ def main():
                      lsmr_iterations=int(r[4]), sm_mhz=r[5], sw_power_cap=bool(r[6])) for r in all_pr.reshape(-1, 7).tolist()]
     sc_all, itn_all, fl_all = smap.read()
     smap.close()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs,
+                     dict(candidate_index=np.arange(lo, lo + len(sc_all), dtype=np.float64), scores=sc_all,
+                          itn=itn_all.astype(np.float64), flags=fl_all.astype(np.float64)),
+                     dict(top_scores=top[0].astype(np.float32), top_index=top[1].astype(np.float64)))
     per_rank_cands = stats["n_candidates"]
 
     # ---- algorithmic bytes of this rank's launches (SURVEY 8d) -----------------------------------------------------

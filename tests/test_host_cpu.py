@@ -323,6 +323,27 @@ def test_bench_split_tail_keeps_the_candidates_and_whole_twist_rows():
     assert [len(c[1]) for c in bench.split_tail(ragged, 2, 600)] == [24] * 4
 
 
+def test_bench_dump_outputs_writes_float_arrays_and_samples_above_the_limit(tmp_path):
+    import bench
+
+    n = 1000
+    per = dict(candidate_index=np.arange(5, 5 + n, dtype=np.float64), scores=np.linspace(0, 1, n, dtype=np.float32))
+    top = dict(top_scores=np.ones(3, np.float32), top_index=np.arange(3, dtype=np.float64))
+    bench.dump_outputs(str(tmp_path / "all"), per, top)
+    for k, v in {**per, **top}.items():
+        got = np.load(tmp_path / "all" / (k + ".npy"))
+        assert got.dtype == v.dtype and np.array_equal(got, v), k
+    limit = 100 * 12 + 3 * 12 + 4 * bench.NPY_HEADER_BYTES  # 100 entries of 12 B, the top-K arrays, 4 headers
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), per, top, limit=limit)
+    idx = np.load(tmp_path / "a" / "candidate_index.npy")
+    assert len(idx) == 100 and np.array_equal(idx, np.load(tmp_path / "b" / "candidate_index.npy"))
+    assert np.all(np.diff(idx) > 0) and np.array_equal(np.load(tmp_path / "a" / "scores.npy"), per["scores"][(idx - 5).astype(int)])
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= limit
+    bench.dump_outputs(str(tmp_path / "c"), per, top, limit=limit - 1)  # one byte less: fewer entries, still inside
+    assert sum(f.stat().st_size for f in (tmp_path / "c").iterdir()) <= limit - 1
+
+
 def test_product_back_project_tables_equal_the_reference_outputs():
     """SURVEY 8(a1): the PRODUCT's host helper (not only the oracle's) against the reference's own outputs
     (tests/golden/backproject.npz, oracle/make_golden.py): coordinate tables and pixel values bit for bit."""

@@ -25,7 +25,8 @@ def test_alias_plugin_mounts_the_module_paths():
 def test_reference_test_file_passes_against_helicon_b200(name):
     path = os.path.join(REF_TESTS, name)
     if not os.path.isfile(path):
-        pytest.skip("oracle/_ref/reference_tests absent (run oracle/build_ref.py where /root/reference exists)")
+        pytest.skip("oracle/_ref/reference_tests absent: copy tests/test_denovo3D_solver.py and "
+                    "tests/test_denovo3D_pipeline.py of jianglab/helicon there (oracle/build_ref.py does it from a checkout)")
     out = subprocess.run([sys.executable, "-m", "pytest", "-q", "-x", "-p", "tests.alias_plugin", "-p", "no:cacheprovider",
                           "--rootdir", REF_TESTS, path], cwd=ROOT, capture_output=True, text=True, timeout=1500)
     tail = out.stdout[-3000:] + out.stderr[-1500:]
