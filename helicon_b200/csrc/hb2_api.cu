@@ -2076,18 +2076,20 @@ static int run_trf(hb2_batch* b, const hb2_solve_options* opt, std::vector<TrfSt
   TD T{};
 #define CKT2(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { tmp.free_all(); return fail(HB2_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_)); } } while (0)
   const size_t nv = (size_t)nc * B.npad, nu = (size_t)b->u_total;
-  double** nvecs[] = {&T.G, &T.D, &T.DH, &T.PH, &T.RH, &T.STEP, &T.V, &T.H, &T.HBAR, &T.XIN, &T.W, &T.UN};
+  double** nvecs[] = {&T.G, &T.D, &T.DH, &T.PH, &T.RH, &T.V, &T.H, &T.HBAR, &T.XIN, &T.W, &T.UN};
   for (double** p : nvecs) CKT2(tmp.alloc(p, nv, true, st));
+  T.W2 = T.HBAR; T.AG = T.H;  // see TD
   B.vtie64 = nullptr;
   if (b->n_tie_views > 0) CKT2(tmp.alloc(&B.vtie64, nv, true, st));
   B.bil_ub64 = nullptr;
   if (b->bilinear) CKT2(tmp.alloc(&B.bil_ub64, nu, true, st));
-  double** mvecs[] = {&T.R, &T.UM, &T.Y, &T.Y2};
+  double** mvecs[] = {&T.R, &T.UM, &T.Y, &T.YP, &T.YAG};
   for (double** p : mvecs) CKT2(tmp.alloc(p, nu, true, st));
   long long max_m = 0;
   for (int c = 0; c < nc; ++c) max_m = std::max<long long>(max_m, (long long)b->h_mdata[c] + b->h_msym[c]);
-  const unsigned gn = cdiv(B.npad, HB2_BLOCK * 4), gm = std::max(1u, cdiv(max_m, HB2_BLOCK * 4));
-  T.red_slots = (int)std::max(gn, gm);
+  const unsigned gn = cdiv(B.npad, TRF_SPAN), gm = std::max(1u, cdiv(max_m, TRF_SPAN));
+  T.gn = (int)gn; T.gm = (int)gm;
+  T.red_slots = (int)(gn + gm);
   CKT2(tmp.alloc(&T.red, (size_t)nc * T.red_slots * TRF_NRED, true, st));
   CKT2(tmp.alloc(&T.st, nc, true, st));
   CKT2(tmp.alloc(&T.nactive, 1, true, st));
@@ -2114,16 +2116,25 @@ static int run_trf(hb2_batch* b, const hb2_solve_options* opt, std::vector<TrfSt
   const double EPS = 2.220446049250313e-16;
   const int lsmr_maxiter = opt->max_iter > 0 ? opt->max_iter : 1000;
   const int max_iter = opt->trf_max_iter > 0 ? opt->trf_max_iter : 200;
-  const dim3 g_n(gn, nc), g_m(gm, nc), g_sym(std::max(1, B.part_us_per_cand), nc);
+  const dim3 g_sym(std::max(1, B.part_us_per_cand), nc);
   const dim3 g_adj(cdiv((long long)B.ndisk * (B.L3P / 4), HB2_BLOCK), nc);
   const size_t sm64 = (size_t)HB2_ADJT_NS * HB2_ADJT_SV * B.K * HB2_BLOCK * sizeof(uint16_t) +
                       (size_t)HB2_ADJT_NS * HB2_ADJT_SV * B.rmax * B.L3P * sizeof(double);
   const unsigned g_fwd = (unsigned)b->nviews * ((B.D2 + HB2_TILE_RAYS - 1) / HB2_TILE_RAYS);
-  const unsigned g_sc = cdiv(nc, 128);
-  auto ew = [&](int op) { k_trf_ew<<<g_n, HB2_BLOCK, 0, st>>>(B, T, op); ++launches; };
-  auto mw = [&](int op) { k_trf_mw<<<g_m, HB2_BLOCK, 0, st>>>(B, T, op); ++launches; };
-  auto red = [&](int nslots, int add, int gate, int start = 0) { k_trf_reduce<<<nc, HB2_BLOCK, 0, st>>>(B, T, nslots, add, gate, start); ++launches; };
-  auto sc = [&](int op) { k_trf_scal<<<g_sc, 128, 0, st>>>(B, T, op, EPS, lsmr_maxiter, max_iter); ++launches; };
+  // pass<OP>() runs an element-wise pass; red(OP, SC) combines its partials and takes the scalar decision SC
+  auto pass = [&](auto op) {
+    constexpr int OP = decltype(op)::value;
+    k_trf_pass<OP><<<dim3(trf_blocks(OP, gn, gm), nc), HB2_BLOCK, 0, st>>>(B, T);
+    ++launches;
+  };
+  auto red = [&](auto op, int sc) {
+    constexpr int OP = decltype(op)::value;
+    k_trf_reduce<<<nc, HB2_BLOCK, 0, st>>>(B, T, (int)trf_blocks(OP, gn, gm), trf_mask(OP), sc, EPS, lsmr_maxiter, max_iter);
+    ++launches;
+  };
+  auto pr = [&](auto op, int sc) { pass(op); red(op, sc); };
+  using std::integral_constant;
+#define OPC(X) integral_constant<int, X>{}
   auto fwd = [&](const double* src, double* dst, int gate) {
     if (B.bt64.nband > 0) {  // float64 instantiation of the band path (bands of half the voxels)
       const dim3 gb(B.bt64.nband, nc), gr(b->max_views, nc);
@@ -2202,50 +2213,45 @@ static int run_trf(hb2_batch* b, const hb2_solve_options* opt, std::vector<TrfSt
     return e;
   };
   // is the unconstrained solution feasible? (lsq_linear.py:328)
-  ew(EW_START); red(gn, 0, 0, 1); sc(SC_START);
+  pr(OPC(EW_START), SC_START);
   int nact = 0;
   CKT2(read_counter(T.nactive, nact));
   outer_iters = 0;
   if (nact > 0) {
-    k_trf_start_apply<<<g_n, HB2_BLOCK, 0, st>>>(B, T); ++launches;
-    fwd(T.W, T.Y, 0); mw(MW_RESID); red(gm, 0, 0); sc(SC_RESID0);
+    pass(OPC(EW_START_APPLY));
+    fwd(T.W, T.Y, 0); pr(OPC(MW_RESID), SC_RESID0);
     adj(T.R, T.G, 0);
     for (int it = 0; it <= max_iter && nact > 0; ++it) {
-      ew(EW_PREP); red(gn, 0, 0); sc(SC_PREP);
+      // scaling, the inner solve's first vector D*(A^T r) (A^T r = G: no adjoint) and the anti-gradient's n-space terms
+      CKT2(cudaMemsetAsync(T.ninner, 0, sizeof(int), st));
+      pr(OPC(EW_PREP), SC_PREP);
       CKT2(read_counter(T.nactive, nact));
       if (nact == 0) break;
       ++outer_iters;
       // inner LSMR on [A D; sqrt(diag_h)] p_h = -[r; 0]   (trf_linear.py:209-216)
-      CKT2(cudaMemsetAsync(T.ninner, 0, sizeof(int), st));
-      adj(T.UM, T.W, 0); ew(EW_INNER_INIT); red(gn, 0, 0); sc(SC_INNER_INIT);
-      ew(EW_INNER_UPD);  // itn == 0: normalise v, h = v, hbar = x = 0, W = D v
+      pass(OPC(EW_INNER_UPD));  // itn == 0: normalise v, h = v, hbar = x = 0, W = D v
       int ninner = 1;
       for (int k = 0; k < lsmr_maxiter && ninner > 0; ++k) {
-        fwd(T.W, T.Y, 1); mw(MW_INNER_U); red(gm, 0, 1);
-        ew(EW_INNER_UN); red(gn, 1, 1); sc(SC_INNER_BETA);
-        adj(T.UM, T.W, 1); ew(EW_INNER_V); red(gn, 0, 1); sc(SC_INNER_ROT);
-        ew(EW_INNER_UPD); red(gn, 0, 1); sc(SC_INNER_TEST);
+        fwd(T.W, T.Y, 1); pr(OPC(NM_INNER_U), SC_INNER_BETA);
+        adj(T.UM, T.W, 1); pr(OPC(EW_INNER_V), SC_INNER_ROT);
+        pr(OPC(EW_INNER_UPD), SC_INNER_TEST);
         if (k % 2 == 1 || k + 1 == lsmr_maxiter) CKT2(read_counter(T.ninner, ninner));
       }
-      // select_step (trf_linear.py:91-144)
-      ew(EW_STEP1); red(gn, 0, 0); sc(SC_STEP1);
-      ew(EW_STEP2); red(gn, 0, 2); sc(SC_STEP2);
-      fwd(T.W, T.Y, 2);
-      ew(EW_LOAD_PH); fwd(T.W, T.Y2, 2);
-      mw(MW_DOTS3); red(gm, 0, 2); sc(SC_SAVE_M);
-      ew(EW_DOTS); red(gn, 0, 2); sc(SC_QUAD);
-      ew(EW_AG); red(gn, 0, 2); sc(SC_SAVE_AG);
-      fwd(T.W, T.Y, 2); mw(MW_DOT_YY); red(gm, 0, 2); sc(SC_AG);
-      // step, predicted cost change, new point, residual, gradient (trf_linear.py:219-243)
-      ew(EW_MKSTEP); red(gn, 0, 0); sc(SC_SAVE_SG);
-      fwd(T.W, T.Y, 0); mw(MW_DOT_YY); red(gm, 0, 0); sc(SC_CC);
-      ew(EW_XUPD);
-      fwd(T.W, T.Y, 0); mw(MW_RESID); red(gm, 0, 0); sc(SC_RESID);
+      // select_step (trf_linear.py:91-144): A*(D*RH), A*(D*PH) (full steps too), A*(-D*D*G)
+      pr(OPC(EW_STEP1), SC_STEP1);
+      pr(OPC(EW_STEP2), SC_STEP2);
+      fwd(T.W, T.Y, 2); fwd(T.W2, T.YP, 0); fwd(T.AG, T.YAG, 2);
+      pr(OPC(MW_DOTS), SC_SELECT);
+      // predicted cost change from the three products, new point, residual, gradient (trf_linear.py:219-243)
+      pr(OPC(NM_STEP), SC_CC);
+      pass(OPC(EW_XUPD));
+      fwd(T.W, T.Y, 0); pr(OPC(MW_RESID), SC_RESID);
       adj(T.R, T.G, 0);
       CKT2(cudaGetLastError());
     }
   }
-  ew(EW_FINAL);
+  pass(OPC(EW_FINAL));
+#undef OPC
   CKT2(cudaGetLastError());
   CKT2(cudaMemcpyAsync(out.data(), T.st, sizeof(TrfState) * nc, cudaMemcpyDeviceToHost, st));
   CKT2(cudaStreamSynchronize(st));

@@ -8,6 +8,8 @@
 #include "hb2_kernels.cuh"
 
 #define TRF_NRED 8  // reduction slots per CTA
+#define TRF_EPT 16  // elements per thread of the element-wise passes
+#define TRF_SPAN (HB2_BLOCK * TRF_EPT)
 
 struct Lsmr64 {  // lsmr.py:197-480, all float64
   double alpha, beta, normb;
@@ -24,7 +26,8 @@ struct TrfState {
   double cost_change;
   double coef_p, coef_r, coef_ag;  // step = D*(coef_p*PH + coef_r*RH + coef_ag*(-GH))
   double acc[TRF_NRED];            // last reduction (sums 0..5, min 6, max 7)
-  double m0, m1, m2, r_value, p_value, ag_n0, ag_n1, ag_min, step_g;
+  double qn[5];                    // n-space dots of build_quadratic_1d / evaluate_quadratic (EW_STEP2)
+  double r_value, p_value, ag_n0, ag_n1, ag_min;
   int active;      // outer loop still running
   int needed;      // bounded branch taken at all
   int status, nit, stop_next, full_step;
@@ -35,10 +38,16 @@ struct TrfState {
 
 struct TD {  // device buffers of the bounded branch
   TrfState* st;
-  double *G, *D, *DH, *PH, *RH, *STEP, *V, *H, *HBAR, *XIN, *W, *UN;  // [nc][npad]
-  double *R, *UM, *Y, *Y2;                                          // rows layout of u (u_total)
+  double *G, *D, *DH, *PH, *RH, *V, *H, *HBAR, *XIN, *W, *UN;  // [nc][npad]
+  // sources of the select_step forwards A*(D*PH) and A*(-D*D*G).  They share storage with HBAR and H, which the
+  // inner solve re-initialises at its first step and which are dead from EW_STEP1 to the next outer iteration.
+  double *W2, *AG;
+  // rows layout of u (u_total).  In select_step Y holds A*(D*RH), YP A*(D*PH) and YAG A*(-D*D*G); the step's A*step
+  // is their combination (no forward of the step itself).
+  double *R, *UM, *Y, *YP, *YAG;
   double* red;      // [nc][red_slots][TRF_NRED]
   int red_slots;
+  int gn, gm;       // CTAs of an n-space / m-space pass (TRF_SPAN elements each)
   int* nactive;
   int* ninner;
 };
@@ -271,57 +280,36 @@ __global__ void __launch_bounds__(HB2_BLOCK) k_adj64(BD B, TD T, const double* _
 }
 
 // ---------------------------------------------------------------------------
-// reductions: each CTA writes TRF_NRED partials to a fixed slot (sums 0..5, min
-// 6, max 7); k_trf_reduce combines a candidate's slots in a fixed order into
-// TrfState::acc (deterministic).
+// reductions: each CTA of a pass writes the partials of the slots its op uses
+// (sums 0..5, min 6, max 7) to a fixed slot of the candidate; k_trf_reduce
+// combines a candidate's slots in a fixed order into TrfState::acc and then takes
+// the candidate's scalar decision.  No atomics, and a candidate's arithmetic does
+// not depend on which other candidates share the batch.
 // ---------------------------------------------------------------------------
-__device__ __forceinline__ double block_minmax_d(double x, bool is_min, double* shd) {
+__device__ __forceinline__ double trf_combine(int k, double a, double b) {
+  return k < 6 ? a + b : (k == 6 ? fmin(a, b) : fmax(a, b));
+}
+__device__ __forceinline__ double trf_identity(int k) { return k < 6 ? 0.0 : (k == 6 ? INFINITY : -INFINITY); }
+
+// block-wide combination of the slots in mask; thread 0 gets the results.  One barrier for all slots.
+__device__ __forceinline__ void trf_block_reduce(double (&v)[TRF_NRED], unsigned mask, double (*shd)[HB2_BLOCK / 32]) {
+  const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
 #pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    double y = __shfl_xor_sync(0xffffffffu, x, o);
-    x = is_min ? fmin(x, y) : fmax(x, y);
+  for (int k = 0; k < TRF_NRED; ++k) {
+    if (!(mask >> k & 1u)) continue;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v[k] = trf_combine(k, v[k], __shfl_xor_sync(0xffffffffu, v[k], o));
+    if (l == 0) shd[k][w] = v[k];
   }
-  int w = threadIdx.x >> 5, l = threadIdx.x & 31;
-  if (l == 0) shd[w] = x;
   __syncthreads();
   if (w == 0) {
-    x = l < HB2_BLOCK / 32 ? shd[l] : (is_min ? INFINITY : -INFINITY);
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      double y = __shfl_xor_sync(0xffffffffu, x, o);
-      x = is_min ? fmin(x, y) : fmax(x, y);
-    }
-  }
-  __syncthreads();
-  return x;
-}
-__device__ __forceinline__ void trf_store_partials(TD T, int c, int slot, double (&v)[TRF_NRED], double* shd) {
+    for (int k = 0; k < TRF_NRED; ++k) {
+      if (!(mask >> k & 1u)) continue;
+      double x = l < HB2_BLOCK / 32 ? shd[k][l] : trf_identity(k);
 #pragma unroll
-  for (int k = 0; k < TRF_NRED; ++k) {
-    double x = k < 6 ? block_sum_d(v[k], shd) : block_minmax_d(v[k], k == 6, shd);
-    if (threadIdx.x == 0) T.red[((size_t)c * T.red_slots + slot) * TRF_NRED + k] = x;
-  }
-}
-__global__ void __launch_bounds__(HB2_BLOCK) k_trf_reduce(BD B, TD T, int nslots, int add, int gate, int start) {
-  const int c = blockIdx.x;
-  __shared__ double shd[HB2_BLOCK / 32];
-  TrfState& S = T.st[c];
-  if (!(start ? (S.needed != 0) : trf_gate(S, gate))) return;
-  double v[TRF_NRED];
-#pragma unroll
-  for (int k = 0; k < TRF_NRED; ++k) v[k] = k < 6 ? 0.0 : (k == 6 ? INFINITY : -INFINITY);
-  for (int s2 = threadIdx.x; s2 < nslots; s2 += HB2_BLOCK) {
-    const double* p = T.red + ((size_t)c * T.red_slots + s2) * TRF_NRED;
-#pragma unroll
-    for (int k = 0; k < 6; ++k) v[k] += p[k];
-    v[6] = fmin(v[6], p[6]); v[7] = fmax(v[7], p[7]);
-  }
-#pragma unroll
-  for (int k = 0; k < TRF_NRED; ++k) {
-    double x = k < 6 ? block_sum_d(v[k], shd) : block_minmax_d(v[k], k == 6, shd);
-    if (threadIdx.x == 0) {
-      if (add) S.acc[k] = k < 6 ? S.acc[k] + x : (k == 6 ? fmin(S.acc[k], x) : fmax(S.acc[k], x));
-      else S.acc[k] = x;
+      for (int o = 16; o > 0; o >>= 1) x = trf_combine(k, x, __shfl_xor_sync(0xffffffffu, x, o));
+      v[k] = x;
     }
   }
 }
@@ -331,147 +319,68 @@ __device__ __forceinline__ double step_to_bound(double x, double s, double lb, d
   return fmax((lb - x) / s, (ub - x) / s);
 }
 
+// passes: n-space (unknowns of the candidate), m-space (its rows), or both in one launch (the first gn CTAs take the
+// n-range, the next gm the m-range)
 enum {
   EW_START = 0,   // reduction: min/max of x_lsq (in_bounds test, lsq_linear.py:328)
+  EW_START_APPLY, // x <- make_strictly_feasible(reflective_transformation(x_lsq), rstep=0.1) ; W = x   (trf_linear.py:150-151)
   EW_PREP,        // Coleman-Li scaling from (x, g): D = sqrt(v), DH = g*dv ; reduction: max |g v|   (trf_linear.py:183-199)
-  EW_INNER_INIT,  // v~ = D*W (W = A^T r, u_n = 0) ; reduction: sum v~^2
-  EW_INNER_UN,    // u~_n = sqrt(DH)*V - alpha*(u~_n*inv_beta) ; reduction: sum u~_n^2
+                  // + first LSMR vector: V = D*G (D*(A^T r), u_n = 0), UN = 0 ; reduction: sum V^2
+                  // + ag = -D*D*G of select_step (it depends on x and g only): its two n-space dots and min step_to_bound(x, ag)
   EW_INNER_V,     // v~ = (D*W + sqrt(DH)*u~_n)*inv_beta - beta*V ; reduction: sum v~^2
   EW_INNER_UPD,   // V = v~/alpha ; hbar, xin, h ; W = D*V ; reduction: sum xin^2
   EW_STEP1,       // PH = -XIN ; reductions: in_bounds(x + D*PH), min step_size_to_bound(x,p), p.g
-  EW_STEP2,       // RH = reflected PH, PH *= p_stride ; W = D*RH ; reduction: min step_size_to_bound(x+p, r)
-  EW_LOAD_PH,     // W = D*PH
-  EW_DOTS,        // n-space dots of build_quadratic_1d / evaluate_quadratic
-  EW_AG,          // W = D*(-GH) ; reductions: dots, min step_size_to_bound(x, ag)
-  EW_MKSTEP,      // STEP = D*(cp*PH + cr*RH - cag*GH) ; W = STEP ; reduction: STEP.G
-  EW_XUPD,        // X = make_strictly_feasible(X + STEP, rstep=0) ; W = X
-  EW_FINAL        // xs = float32(X)   (SLR:270)
+  EW_STEP2,       // RH = reflected PH, PH *= p_stride ; W = D*RH, W2 = D*PH, AG = -D*D*G ; reductions: min step_size_to_bound(x+p, r),
+                  // n-space dots of build_quadratic_1d / evaluate_quadratic.  Full-step candidates: W2 = D*PH only.
+  EW_XUPD,        // X = make_strictly_feasible(X + step, rstep=0) ; W = X
+  EW_FINAL,       // xs = float32(X)   (SLR:270)
+  MW_RESID,       // R = A x - b ; u~_m = R (right-hand side of the next inner solve) ; sum R^2
+  MW_DOTS,        // dots of Y = A_h r_h, YP = A_h p_h, YAG = A_h ag_h
+  NM_INNER_U,     // n: u~_n = sqrt(DH)*V - alpha*(u~_n*inv_beta) ; m: u~_m = Y - alpha*(u~_m*inv_beta) ; sum of both squared
+  NM_STEP         // n: step.g with step = D*(cp*PH + cr*RH - cag*D*G) ; m: |A step|^2, A step = cp*YP + cr*Y + cag*YAG
 };
-
-__global__ void __launch_bounds__(HB2_BLOCK) k_trf_ew(BD B, TD T, int op) {
-  const int c = blockIdx.y;
-  __shared__ double shd[HB2_BLOCK / 32];
-  const TrfState& S = T.st[c];
-  bool act;
-  if (op == EW_START || op == EW_FINAL) act = S.needed != 0;
-  else if (op == EW_INNER_UPD) act = S.active && (S.in.active || S.in.itn == 0);
-  else if (op == EW_INNER_UN || op == EW_INNER_V) act = trf_gate(S, 1);
-  else if (op == EW_STEP2 || op == EW_LOAD_PH || op == EW_DOTS || op == EW_AG) act = trf_gate(S, 2);
-  else act = trf_gate(S, 0);
-  if (op == EW_INNER_V && S.in.skip_adj) act = false;
-  if (!act) return;
-  const size_t o = (size_t)c * B.npad;
-  double* X = B.x + o;
-  double red[TRF_NRED] = {0, 0, 0, 0, 0, 0, INFINITY, -INFINITY};
-  const double lb = S.lb, ub = S.ub;
-  for (int i = blockIdx.x * HB2_BLOCK * 4 + threadIdx.x, qq = 0; qq < 4; ++qq, i += HB2_BLOCK) {
-    if (i >= B.npad || (i % B.L3P) >= B.L3) continue;  // padded slices are not unknowns
-    const size_t e = o + i;
-    switch (op) {
-      case EW_START: {
-        double y = X[i];
-        red[6] = fmin(red[6], y); red[7] = fmax(red[7], y);
-      } break;
-      case EW_PREP: {
-        double x = X[i], g = T.G[e], v = 1.0, dv = 0.0;
-        if (g < 0) { v = ub - x; dv = -1.0; }
-        if (g > 0) { v = x - lb; dv = 1.0; }
-        T.D[e] = sqrt(v); T.DH[e] = g * dv;
-        red[7] = fmax(red[7], fabs(g * v));
-      } break;
-      case EW_INNER_INIT: {
-        double vt = T.D[e] * T.W[e];
-        T.UN[e] = 0.0; T.V[e] = vt; red[0] += vt * vt;
-      } break;
-      case EW_INNER_UN: {
-        double un = sqrt(T.DH[e]) * T.V[e] - S.in.alpha * (T.UN[e] * S.in.inv_beta);
-        T.UN[e] = un; red[0] += un * un;
-      } break;
-      case EW_INNER_V: {
-        double vt = (T.D[e] * T.W[e] + sqrt(T.DH[e]) * T.UN[e]) * S.in.inv_beta - S.in.beta * T.V[e];
-        T.V[e] = vt; red[0] += vt * vt;
-      } break;
-      case EW_INNER_UPD: {
-        double vn = T.V[e];
-        if (S.in.itn == 0 || !S.in.skip_adj) { vn *= S.in.inv_alpha; T.V[e] = vn; }
-        if (S.in.itn == 0) { T.H[e] = vn; T.HBAR[e] = 0.0; T.XIN[e] = 0.0; }
-        else {
-          double ho = T.H[e];
-          double hb = T.HBAR[e] * S.in.cf_hbar + ho;
-          T.HBAR[e] = hb;
-          double xn = T.XIN[e] + S.in.cf_x * hb;
-          T.XIN[e] = xn;
-          T.H[e] = ho * S.in.cf_h + vn;
-          red[0] += xn * xn;
-        }
-        T.W[e] = T.D[e] * vn;
-      } break;
-      case EW_STEP1: {
-        double ph = -T.XIN[e];
-        T.PH[e] = ph;
-        double x = X[i], p = T.D[e] * ph, xp = x + p;
-        red[6] = fmin(red[6], fmin(xp - lb, ub - xp));
-        red[5] += p * T.G[e];
-        red[7] = fmax(red[7], -step_to_bound(x, p, lb, ub));
-      } break;
-      case EW_STEP2: {
-        double ph = T.PH[e], x = X[i], d = T.D[e];
-        double p = d * ph;
-        double st = step_to_bound(x, p, lb, ub);
-        double rh = (st == S.p_stride && p != 0.0) ? -ph : ph;  // hits -> reflect (trf_linear.py:97-99)
-        T.RH[e] = rh;
-        T.PH[e] = ph * S.p_stride;
-        double xb = x + p * S.p_stride, r = d * rh;
-        red[7] = fmax(red[7], -step_to_bound(xb, r, lb, ub));
-        T.W[e] = r;
-      } break;
-      case EW_LOAD_PH: T.W[e] = T.D[e] * T.PH[e]; break;
-      case EW_DOTS: {
-        double ph = T.PH[e], rh = T.RH[e], dh = T.DH[e], gh = T.D[e] * T.G[e];
-        red[0] += rh * dh * rh; red[1] += gh * rh; red[2] += ph * dh * rh; red[3] += gh * ph; red[4] += ph * dh * ph;
-      } break;
-      case EW_AG: {
-        double d = T.D[e], g = T.G[e], gh = d * g, agh = -gh, ag = d * agh;
-        red[0] += agh * T.DH[e] * agh; red[1] += gh * agh;
-        red[7] = fmax(red[7], -step_to_bound(X[i], ag, lb, ub));
-        T.W[e] = ag;
-      } break;
-      case EW_MKSTEP: {
-        double d = T.D[e];
-        double s2 = d * (S.coef_p * T.PH[e] + S.coef_r * T.RH[e] - S.coef_ag * (d * T.G[e]));
-        T.STEP[e] = s2; T.W[e] = s2; red[0] += s2 * T.G[e];
-      } break;
-      case EW_XUPD: {
-        double x = X[i];
-        if (S.cost_change >= 0) {  // else: scipy's backtracking() hands back the OLD x (trf_linear.py:69-88)
-          x = x + T.STEP[e];
-          if (x <= lb) x = nextafter(lb, ub);
-          if (x >= ub) x = nextafter(ub, lb);
-          if (x < lb || x > ub) x = 0.5 * (lb + ub);
-          X[i] = x;
-        }
-        T.W[e] = x;
-      } break;
-      case EW_FINAL: B.xs[e] = (float)X[i]; break;
-    }
-  }
-  if (op == EW_LOAD_PH || op == EW_XUPD || op == EW_FINAL) return;
-  trf_store_partials(T, c, blockIdx.x, red, shd);
+__host__ __device__ constexpr bool trf_has_n(int op) { return op < MW_RESID || op >= NM_INNER_U; }
+__host__ __device__ constexpr bool trf_has_m(int op) { return op >= MW_RESID; }
+__host__ __device__ constexpr unsigned trf_mask(int op) {  // reduction slots an op fills
+  return op == EW_START ? 0xC0u : op == EW_PREP ? 0xC7u : op == EW_STEP1 ? 0xE0u : op == EW_STEP2 ? 0x9Fu
+       : op == MW_DOTS ? 0x0Fu : op == NM_STEP ? 0x03u
+       : (op == EW_START_APPLY || op == EW_XUPD || op == EW_FINAL) ? 0u : 0x01u;
+}
+__host__ __device__ constexpr unsigned trf_blocks(int op, unsigned gn, unsigned gm) {
+  return (trf_has_n(op) ? gn : 0u) + (trf_has_m(op) ? gm : 0u);
 }
 
-// x <- make_strictly_feasible(reflective_transformation(x_lsq), rstep=0.1)  (trf_linear.py:150-151)
-__global__ void __launch_bounds__(HB2_BLOCK) k_trf_start_apply(BD B, TD T) {
-  const int c = blockIdx.y;
-  const TrfState& S = T.st[c];
-  if (!S.active) return;
-  double* X = B.x + (size_t)c * B.npad;
-  const double lb = S.lb, ub = S.ub, d = ub - lb;
-  for (int i = blockIdx.x * HB2_BLOCK * 4 + threadIdx.x, qq = 0; qq < 4; ++qq, i += HB2_BLOCK) {
-    if (i >= B.npad || (i % B.L3P) >= B.L3) continue;
+// gate: 0 outer-active, 1 inner-active, 2 outer-active and reflective part needed
+__device__ __forceinline__ bool trf_pass_active(const TrfState& S, int op) {
+  switch (op) {
+    case EW_START: case EW_FINAL: return S.needed != 0;
+    case EW_START_APPLY: return S.active != 0;
+    case EW_INNER_UPD: return S.active && (S.in.active || S.in.itn == 0);
+    case NM_INNER_U: return trf_gate(S, 1);
+    case EW_INNER_V: return trf_gate(S, 1) && !S.in.skip_adj;
+    case MW_DOTS: return trf_gate(S, 2);
+    default: return trf_gate(S, 0);
+  }
+}
+
+// the step of trf_linear.py:219-225 rebuilt from PH, RH, D and G (it is never stored)
+__device__ __forceinline__ double trf_step(const TrfState& S, const TD& T, size_t e) {
+  const double d = T.D[e];
+  return d * (S.coef_p * T.PH[e] + S.coef_r * T.RH[e] - S.coef_ag * (d * T.G[e]));
+}
+
+template <int OP>
+__device__ __forceinline__ void trf_n_elem(const BD& B, const TD& T, const TrfState& S, double* X, int i, size_t e,
+                                           double (&red)[TRF_NRED]) {
+  const double lb = S.lb, ub = S.ub;
+  if constexpr (OP == EW_START) {
     double y = X[i];
-    double t = fmod(y - lb, 2 * d);
-    if (t < 0) t += 2 * d;  // np.remainder takes the sign of the divisor (common.py:535)
-    double x = lb + fmin(t, 2 * d - t);
+    red[6] = fmin(red[6], y); red[7] = fmax(red[7], y);
+  } else if constexpr (OP == EW_START_APPLY) {
+    const double y = X[i], dd = ub - lb;
+    double t = fmod(y - lb, 2 * dd);
+    if (t < 0) t += 2 * dd;  // np.remainder takes the sign of the divisor (common.py:535)
+    double x = lb + fmin(t, 2 * dd - t);
     // make_strictly_feasible(rstep=0.1): common.py:440-464 with find_active_constraints (:401-437)
     double ld = x - lb, udist = ub - x;
     double lth = 0.1 * fmax(1.0, fabs(lb)), uth = 0.1 * fmax(1.0, fabs(ub));
@@ -480,49 +389,152 @@ __global__ void __launch_bounds__(HB2_BLOCK) k_trf_start_apply(BD B, TD T) {
     if (ua) x = ub - 0.1 * fmax(1.0, fabs(ub));
     if (x < lb || x > ub) x = 0.5 * (lb + ub);
     X[i] = x;
-    T.W[(size_t)c * B.npad + i] = x;
+    T.W[e] = x;
+  } else if constexpr (OP == EW_PREP) {
+    double x = X[i], g = T.G[e], v = 1.0, dv = 0.0;
+    if (g < 0) { v = ub - x; dv = -1.0; }
+    if (g > 0) { v = x - lb; dv = 1.0; }
+    const double d = sqrt(v), dh = g * dv;
+    T.D[e] = d; T.DH[e] = dh;
+    red[7] = fmax(red[7], fabs(g * v));
+    const double gh = d * g;  // = D*(A^T r): the inner solve's first v (before 1/beta)
+    T.UN[e] = 0.0; T.V[e] = gh; red[0] += gh * gh;
+    const double agh = -gh, ag = d * agh;
+    red[1] += agh * dh * agh; red[2] += gh * agh;
+    red[6] = fmin(red[6], step_to_bound(x, ag, lb, ub));
+  } else if constexpr (OP == EW_INNER_V) {
+    double vt = (T.D[e] * T.W[e] + sqrt(T.DH[e]) * T.UN[e]) * S.in.inv_beta - S.in.beta * T.V[e];
+    T.V[e] = vt; red[0] += vt * vt;
+  } else if constexpr (OP == EW_INNER_UPD) {
+    double vn = T.V[e];
+    if (S.in.itn == 0 || !S.in.skip_adj) { vn *= S.in.inv_alpha; T.V[e] = vn; }
+    if (S.in.itn == 0) { T.H[e] = vn; T.HBAR[e] = 0.0; T.XIN[e] = 0.0; }
+    else {
+      double ho = T.H[e];
+      double hb = T.HBAR[e] * S.in.cf_hbar + ho;
+      T.HBAR[e] = hb;
+      double xn = T.XIN[e] + S.in.cf_x * hb;
+      T.XIN[e] = xn;
+      T.H[e] = ho * S.in.cf_h + vn;
+      red[0] += xn * xn;
+    }
+    T.W[e] = T.D[e] * vn;
+  } else if constexpr (OP == EW_STEP1) {
+    double ph = -T.XIN[e];
+    T.PH[e] = ph;
+    double x = X[i], p = T.D[e] * ph, xp = x + p;
+    red[6] = fmin(red[6], fmin(xp - lb, ub - xp));
+    red[5] += p * T.G[e];
+    red[7] = fmax(red[7], -step_to_bound(x, p, lb, ub));
+  } else if constexpr (OP == EW_STEP2) {
+    const double ph = T.PH[e], d = T.D[e];
+    if (S.full_step) { T.W2[e] = d * ph; return; }
+    const double x = X[i], p = d * ph;
+    const double st = step_to_bound(x, p, lb, ub);
+    const double rh = (st == S.p_stride && p != 0.0) ? -ph : ph;  // hits -> reflect (trf_linear.py:97-99)
+    const double phs = ph * S.p_stride;
+    T.RH[e] = rh; T.PH[e] = phs;
+    const double xb = x + p * S.p_stride, r = d * rh;
+    red[7] = fmax(red[7], -step_to_bound(xb, r, lb, ub));
+    T.W[e] = r; T.W2[e] = d * phs;
+    const double dh = T.DH[e], gh = d * T.G[e];
+    red[0] += rh * dh * rh; red[1] += gh * rh; red[2] += phs * dh * rh; red[3] += gh * phs; red[4] += phs * dh * phs;
+    T.AG[e] = d * -gh;
+  } else if constexpr (OP == EW_XUPD) {
+    double x = X[i];
+    if (S.cost_change >= 0) {  // else: scipy's backtracking() hands back the OLD x (trf_linear.py:69-88)
+      x = x + trf_step(S, T, e);
+      if (x <= lb) x = nextafter(lb, ub);
+      if (x >= ub) x = nextafter(ub, lb);
+      if (x < lb || x > ub) x = 0.5 * (lb + ub);
+      X[i] = x;
+    }
+    T.W[e] = x;
+  } else if constexpr (OP == EW_FINAL) {
+    B.xs[e] = (float)X[i];
+  } else if constexpr (OP == NM_INNER_U) {
+    double un = sqrt(T.DH[e]) * T.V[e] - S.in.alpha * (T.UN[e] * S.in.inv_beta);
+    T.UN[e] = un; red[0] += un * un;
+  } else if constexpr (OP == NM_STEP) {
+    red[1] += trf_step(S, T, e) * T.G[e];
   }
 }
 
-// m-space kernels (rows of candidate c live at [cand_uoff, + mdata + msym)) ---------
-enum { MW_RESID = 0, MW_INNER_U, MW_DOTS3, MW_DOT_YY };
-__global__ void __launch_bounds__(HB2_BLOCK) k_trf_mw(BD B, TD T, int op) {
+template <int OP>
+__device__ __forceinline__ void trf_m_elem(const BD& B, const TD& T, const TrfState& S, int c, long long r, size_t e,
+                                           double (&red)[TRF_NRED]) {
+  if constexpr (OP == MW_RESID) {
+    double bb = r < B.cand_mdata[c] ? (double)B.b[e] : 0.0;
+    double res = T.Y[e] - bb;
+    T.R[e] = res; T.UM[e] = res; red[0] += res * res;
+  } else if constexpr (OP == NM_INNER_U) {
+    double un = T.Y[e] - S.in.alpha * (T.UM[e] * S.in.inv_beta);
+    T.UM[e] = un; red[0] += un * un;
+  } else if constexpr (OP == MW_DOTS) {
+    double v1 = T.Y[e], u1 = T.YP[e], a = T.YAG[e];
+    red[0] += v1 * v1; red[1] += u1 * v1; red[2] += u1 * u1; red[3] += a * a;
+  } else if constexpr (OP == NM_STEP) {  // at most two coefficients are non-zero; the others' vectors are not read
+    double v = 0.0;
+    if (S.coef_p != 0.0) v += S.coef_p * T.YP[e];
+    if (S.coef_r != 0.0) v += S.coef_r * T.Y[e];
+    if (S.coef_ag != 0.0) v += S.coef_ag * T.YAG[e];
+    red[0] += v * v;
+  }
+}
+
+template <int OP>
+__global__ void __launch_bounds__(HB2_BLOCK) k_trf_pass(BD B, TD T) {
   const int c = blockIdx.y;
-  __shared__ double shd[HB2_BLOCK / 32];
   const TrfState& S = T.st[c];
-  bool act = op == MW_INNER_U ? trf_gate(S, 1) : (op == MW_DOTS3 ? trf_gate(S, 2) : trf_gate(S, 0));
-  if (!act) return;
-  const long long m = (long long)B.cand_mdata[c] + B.cand_msym[c];
-  const size_t o = (size_t)B.cand_uoff[c];
-  double red[TRF_NRED] = {0, 0, 0, 0, 0, 0, INFINITY, -INFINITY};
-  for (long long r = (long long)blockIdx.x * HB2_BLOCK * 4 + threadIdx.x, qq = 0; qq < 4; ++qq, r += HB2_BLOCK) {
-    if (r >= m) continue;
-    const size_t e = o + r;
-    switch (op) {
-      case MW_RESID: {  // R = A x - b ; u~_m = R (right-hand side of the next inner solve) ; sum R^2
-        double bb = r < B.cand_mdata[c] ? (double)B.b[e] : 0.0;
-        double res = T.Y[e] - bb;
-        T.R[e] = res; T.UM[e] = res; red[0] += res * res;
-      } break;
-      case MW_INNER_U: {
-        double un = T.Y[e] - S.in.alpha * (T.UM[e] * S.in.inv_beta);
-        T.UM[e] = un; red[0] += un * un;
-      } break;
-      case MW_DOTS3: {  // Y = A_h r_h, Y2 = A_h p_h
-        double v1 = T.Y[e], u1 = T.Y2[e];
-        red[0] += v1 * v1; red[1] += u1 * v1; red[2] += u1 * u1;
-      } break;
-      case MW_DOT_YY: { double v = T.Y[e]; red[0] += v * v; } break;
+  if (!trf_pass_active(S, OP)) return;
+  double red[TRF_NRED];
+#pragma unroll
+  for (int k = 0; k < TRF_NRED; ++k) red[k] = trf_identity(k);
+  if (trf_has_n(OP) && (!trf_has_m(OP) || (int)blockIdx.x < T.gn)) {
+    const size_t o = (size_t)c * B.npad;
+    double* X = B.x + o;
+    const int i0 = blockIdx.x * TRF_SPAN + threadIdx.x;
+#pragma unroll 4
+    for (int k = 0; k < TRF_EPT; ++k) {
+      const int i = i0 + k * HB2_BLOCK;
+      if (i >= B.npad || (i % B.L3P) >= B.L3) continue;  // padded slices are not unknowns
+      trf_n_elem<OP>(B, T, S, X, i, o + i, red);
+    }
+  } else if (trf_has_m(OP)) {
+    const long long m = (long long)B.cand_mdata[c] + B.cand_msym[c];
+    const size_t o = (size_t)B.cand_uoff[c];
+    const long long r0 = (long long)(blockIdx.x - (trf_has_n(OP) ? T.gn : 0)) * TRF_SPAN + threadIdx.x;
+#pragma unroll 4
+    for (int k = 0; k < TRF_EPT; ++k) {
+      const long long r = r0 + (long long)k * HB2_BLOCK;
+      if (r >= m) continue;
+      trf_m_elem<OP>(B, T, S, c, r, o + r, red);
     }
   }
-  trf_store_partials(T, c, blockIdx.x, red, shd);
+  constexpr unsigned mask = trf_mask(OP);
+  if constexpr (mask != 0) {
+    __shared__ double shd[TRF_NRED][HB2_BLOCK / 32];
+    trf_block_reduce(red, mask, shd);
+    if (threadIdx.x == 0) {
+      double* dst = T.red + ((size_t)c * T.red_slots + blockIdx.x) * TRF_NRED;
+#pragma unroll
+      for (int k = 0; k < TRF_NRED; ++k)
+        if (mask >> k & 1u) dst[k] = red[k];
+    }
+  }
 }
 
-// scalar decisions: one thread per candidate, reads TrfState::acc ---------------------
+// scalar decisions: thread 0 of k_trf_reduce, after the candidate's partials are combined into TrfState::acc ------
 enum {
-  SC_START = 0, SC_RESID0, SC_PREP, SC_INNER_INIT, SC_INNER_BETA, SC_INNER_ROT, SC_INNER_TEST, SC_STEP1, SC_STEP2,
-  SC_SAVE_M, SC_QUAD, SC_SAVE_AG, SC_AG, SC_SAVE_SG, SC_CC, SC_RESID
+  SC_START = 0, SC_RESID0, SC_PREP, SC_INNER_BETA, SC_INNER_ROT, SC_INNER_TEST, SC_STEP1, SC_STEP2, SC_SELECT, SC_CC,
+  SC_RESID
 };
+__device__ __forceinline__ bool trf_scal_active(const TrfState& S, int op) {
+  if (op == SC_START) return S.needed != 0;
+  if (op == SC_INNER_BETA || op == SC_INNER_ROT || op == SC_INNER_TEST) return trf_gate(S, 1);
+  if (op == SC_STEP2 || op == SC_SELECT) return trf_gate(S, 2);
+  return trf_gate(S, 0);
+}
 __device__ __forceinline__ void min_quadratic_1d(double a, double b, double lo, double hi, double c, double& t, double& y) {
   // common.py:302-322
   double tt[3] = {lo, hi, 0};
@@ -537,14 +549,7 @@ __device__ __forceinline__ void min_quadratic_1d(double a, double b, double lo, 
     if (yy < y) { y = yy; t = tt[k]; }  // np.argmin keeps the first minimum
   }
 }
-__global__ void k_trf_scal(BD B, TD T, int op, double eps, int lsmr_maxiter, int max_iter) {
-  const int c = blockIdx.x * blockDim.x + threadIdx.x;
-  if (c >= B.nc) return;
-  TrfState& S = T.st[c];
-  if (op == SC_START) { if (!S.needed) return; }
-  else if (op == SC_INNER_BETA || op == SC_INNER_ROT || op == SC_INNER_TEST) { if (!trf_gate(S, 1)) return; }
-  else if (op == SC_STEP2 || op == SC_SAVE_M || op == SC_QUAD || op == SC_SAVE_AG || op == SC_AG) { if (!trf_gate(S, 2)) return; }
-  else if (!trf_gate(S, 0)) return;
+__device__ void trf_scalar(const TD& T, TrfState& S, int op, double eps, int lsmr_maxiter, int max_iter) {
   const double* r = S.acc;
   switch (op) {
     case SC_START: {
@@ -564,16 +569,13 @@ __global__ void k_trf_scal(BD B, TD T, int op, double eps, int lsmr_maxiter, int
       double eta = 1e-2 * fmin(0.5, S.g_norm);
       S.lsmr_tol = fmax(eps, fmin(0.1, eta * S.g_norm));
       S.theta = 1 - fmin(0.005, S.g_norm);
-      S.in.beta = sqrt(2 * S.cost);
-      S.in.inv_beta = S.in.beta > 0 ? 1.0 / S.in.beta : 0.0;
-      S.in.itn = 0; S.in.active = 1; S.in.skip_adj = 0; S.in.alpha = 0; S.full_step = 0;
-    } break;
-    case SC_INNER_INIT: {  // V holds D*(A^T r) (not yet divided by beta)
-      double nv = sqrt(r[0]);
-      double beta = S.in.beta;
+      S.full_step = 0;
+      // inner LSMR on [A D; sqrt(diag_h)] p_h = -[r; 0]: V holds D*(A^T r) (not yet divided by beta)
+      const double beta = sqrt(2 * S.cost), nv = sqrt(r[0]);
       lsmr64_init_(S.in, nv * (beta > 0 ? 1.0 / beta : 0.0), beta);
       S.in.inv_alpha = nv > 0 ? 1.0 / nv : 1.0;
       if (S.in.active) atomicAdd(T.ninner, 1);
+      S.ag_n0 = r[1]; S.ag_n1 = r[2]; S.ag_min = r[6];  // ag = -D*D*G (select_step)
     } break;
     case SC_INNER_BETA: {
       S.in.beta = sqrt(r[0]);
@@ -595,20 +597,21 @@ __global__ void k_trf_scal(BD B, TD T, int op, double eps, int lsmr_maxiter, int
       double rsu = -r[7];
       S.r_stride_l = (1 - S.theta) * rsu;
       S.r_stride_u = rsu * S.theta;
+      for (int k = 0; k < 5; ++k) S.qn[k] = r[k];
     } break;
-    case SC_SAVE_M: S.m0 = r[0]; S.m1 = r[1]; S.m2 = r[2]; break;
-    case SC_QUAD: {  // build_quadratic_1d(A_h, g_h, r_h, s0=p_h, diag=diag_h), common.py:251-299
-      double a = 0.5 * (S.m0 + r[0]);
-      double b = r[1] + S.m1 + r[2];
-      double cc = 0.5 * S.m2 + r[3] + 0.5 * r[4];
+    case SC_SELECT: {
+      // build_quadratic_1d(A_h, g_h, r_h, s0=p_h, diag=diag_h), common.py:251-299
+      const double* q = S.qn;
+      const double m0 = r[0], m1 = r[1], m2 = r[2];
+      double a = 0.5 * (m0 + q[0]);
+      double b = q[1] + m1 + q[2];
+      double cc = 0.5 * m2 + q[3] + 0.5 * q[4];
       if (S.r_stride_u > 0) min_quadratic_1d(a, b, S.r_stride_l, S.r_stride_u, cc, S.r_stride, S.r_value);
       else { S.r_value = INFINITY; S.r_stride = 0; }
       double th = S.theta;  // p_h *= theta ; evaluate_quadratic(A_h, g_h, p_h, diag_h)
-      S.p_value = 0.5 * (th * th * S.m2 + th * th * r[4]) + th * r[3];
-    } break;
-    case SC_SAVE_AG: S.ag_n0 = r[0]; S.ag_n1 = r[1]; S.ag_min = -r[7]; break;
-    case SC_AG: {
-      double a = 0.5 * (r[0] + S.ag_n0), b = S.ag_n1;
+      S.p_value = 0.5 * (th * th * m2 + th * th * q[4]) + th * q[3];
+      // anti-gradient step
+      a = 0.5 * (r[3] + S.ag_n0); b = S.ag_n1;
       double ag_value;
       min_quadratic_1d(a, b, 0.0, S.ag_min * S.theta, 0.0, S.ag_stride, ag_value);
       S.ag_value = ag_value;
@@ -616,9 +619,8 @@ __global__ void k_trf_scal(BD B, TD T, int op, double eps, int lsmr_maxiter, int
       else if (S.r_value < S.p_value && S.r_value < ag_value) { S.coef_p = 1.0; S.coef_r = S.r_stride; S.coef_ag = 0; }
       else { S.coef_p = 0; S.coef_r = 0; S.coef_ag = S.ag_stride; }
     } break;
-    case SC_SAVE_SG: S.step_g = r[0]; break;
     case SC_CC: {
-      S.cost_change = -(0.5 * r[0] + S.step_g);  // -evaluate_quadratic(A, g, step)
+      S.cost_change = -(0.5 * r[0] + r[1]);  // -evaluate_quadratic(A, g, step)
       if (S.nit <= 24) {
         double* t = S.trace[S.nit - 1];
         t[2] = S.in.itn;
@@ -630,5 +632,30 @@ __global__ void k_trf_scal(BD B, TD T, int op, double eps, int lsmr_maxiter, int
       if (S.cost_change < S.tol * S.cost) { S.status = 2; S.stop_next = 1; }
       S.cost = 0.5 * r[0];
     } break;
+  }
+}
+
+// one CTA per candidate: combine the nslots partials of the slots in mask in a fixed order, then decide (op)
+__global__ void __launch_bounds__(HB2_BLOCK) k_trf_reduce(BD B, TD T, int nslots, unsigned mask, int op, double eps,
+                                                          int lsmr_maxiter, int max_iter) {
+  const int c = blockIdx.x;
+  __shared__ double shd[TRF_NRED][HB2_BLOCK / 32];
+  TrfState& S = T.st[c];
+  if (!trf_scal_active(S, op)) return;
+  double v[TRF_NRED];
+#pragma unroll
+  for (int k = 0; k < TRF_NRED; ++k) v[k] = trf_identity(k);
+  for (int s2 = threadIdx.x; s2 < nslots; s2 += HB2_BLOCK) {
+    const double* p = T.red + ((size_t)c * T.red_slots + s2) * TRF_NRED;
+#pragma unroll
+    for (int k = 0; k < TRF_NRED; ++k)
+      if (mask >> k & 1u) v[k] = trf_combine(k, v[k], p[k]);
+  }
+  trf_block_reduce(v, mask, shd);
+  if (threadIdx.x == 0) {
+#pragma unroll
+    for (int k = 0; k < TRF_NRED; ++k)
+      if (mask >> k & 1u) S.acc[k] = v[k];
+    trf_scalar(T, S, op, eps, lsmr_maxiter, max_iter);
   }
 }
