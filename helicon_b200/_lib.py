@@ -24,6 +24,7 @@ HB2_FLAG_TIE_Z = 2
 HB2_FLAG_BOUNDED = 4
 HB2_FLAG_NO_ROWS = 8
 HB2_FLAG_TIE_Z_EXACT = 16
+HB2_FLAG_NOT_CONVERGED = 32
 
 
 class Geometry(C.Structure):
@@ -55,6 +56,16 @@ class SolveOptions(C.Structure):
         ("check_every", C.c_int32), ("clip_pred", C.c_int32), ("trf_max_iter", C.c_int32), ("trf_tol", C.c_double),
         ("fixed_iters", C.c_int32), ("profile", C.c_int32), ("norm_mode", C.c_int32),
     ]
+
+
+class ModelOptions(C.Structure):
+    _fields_ = [
+        ("kind", C.c_int32), ("alpha", C.c_double), ("l1_ratio", C.c_double), ("gap_factor", C.c_double),
+        ("max_iter", C.c_int32), ("check_every", C.c_int32), ("clip_pred", C.c_int32), ("power_start", C.c_void_p),
+    ]
+
+
+MODEL_ENET, MODEL_RIDGE = 0, 1
 
 
 class SymmParams(C.Structure):
@@ -105,6 +116,7 @@ EXPORTS = [
     "hb2_batch_bilinear_sym_export",
     "hb2_scoremap_create", "hb2_scoremap_destroy", "hb2_scoremap_device_ptr", "hb2_batch_scatter_scores",
     "hb2_scoremap_merge", "hb2_scoremap_topk", "hb2_scoremap_read", "hb2_scoremap_restore",
+    "hb2_batch_set_real_rows", "hb2_batch_solve_model", "hb2_batch_model_info", "hb2_batch_apply_all",
 ]
 
 _lib = None
@@ -164,6 +176,10 @@ def load():
     lib.hb2_batch_get_x.argtypes = [vp, i32, vp]
     lib.hb2_batch_timing.argtypes = [vp, vp]
     lib.hb2_batch_trf_trace.argtypes = [vp, i32, vp, i32]
+    lib.hb2_batch_set_real_rows.argtypes = [vp, i32, vp, i64]
+    lib.hb2_batch_solve_model.argtypes = [vp, P(ModelOptions), vp]
+    lib.hb2_batch_model_info.argtypes = [vp, i32, vp]
+    lib.hb2_batch_apply_all.argtypes = [vp, i32, vp, vp]
     lib.hb2_helical_symmetrize.argtypes = [vp, P(SymmParams), vp, vp, vp, vp, vp, vp, i32, vp, vp, vp, vp, C.c_int, vp]
     lib.hb2_lsmr_scalar_step.argtypes = [vp, C.c_int, C.c_float, C.c_float, f64, f64, f64, f64, C.c_int, P(C.c_float), P(C.c_float), P(C.c_float), vp]
     lib.hb2_scoremap_create.argtypes = [P(vp), i64, C.c_int]

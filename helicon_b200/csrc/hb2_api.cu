@@ -8,6 +8,7 @@
 #include "hb2_adj_tile.cuh"
 #include "hb2_explicit.cuh"
 #include "hb2_bilinear.cuh"
+#include "hb2_model.cuh"
 
 #include <cub/cub.cuh>
 #include <nvtx3/nvToolsExt.h>
@@ -288,6 +289,10 @@ struct hb2_batch {
   int* h_nactive = nullptr;  // pinned
   double timing[16] = {0};
   std::vector<TrfState> last_trf;
+  // model solves (hb2_batch_solve_model): real-row masks [u_total] and the last fit per candidate (4 values each)
+  uint8_t* d_real = nullptr;
+  std::vector<uint8_t> real_set;
+  std::vector<double> mdl_info;
   std::vector<cudaEvent_t> ev_pool;
   std::vector<std::pair<int, int>> ev_used;  // (class, index of start event)
   size_t ev_next = 0;
@@ -2408,6 +2413,264 @@ extern "C" int hb2_batch_solve(hb2_batch* b, const hb2_solve_options* opt, hb2_r
   }
   b->solved = true;
   b->last_trf = trf;
+  return HB2_OK;
+}
+
+// ---------------------------------------------------------------------------
+// ElasticNet / Lasso / Ridge for every candidate of the batch (hb2_model.cuh)
+// ---------------------------------------------------------------------------
+extern "C" int hb2_batch_set_real_rows(hb2_batch* b, int32_t c, const uint8_t* real, int64_t m) {
+  if (!b || !b->created || !real || c < 0 || c >= b->B.nc) return fail(HB2_ERR_ARG, "bad argument");
+  if (m != (int64_t)b->h_mdata[c] + b->h_msym[c]) return fail(HB2_ERR_ARG, "real-row mask: m is not the candidate's padded row count");
+  CK(cudaSetDevice(b->P->device));
+  if (!b->d_real) {
+    CK(b->pool.alloc(&b->d_real, (size_t)b->u_total, true, b->stream));
+    b->real_set.assign(b->B.nc, 0);
+  }
+  CK(cudaMemcpyAsync(b->d_real + b->h_uoff[c], real, (size_t)m, cudaMemcpyHostToDevice, b->stream));
+  CK(cudaStreamSynchronize(b->stream));  // the host buffer may go away after the call
+  b->real_set[c] = 1;
+  return HB2_OK;
+}
+
+extern "C" int hb2_batch_apply_all(hb2_batch* b, int32_t adjoint, const float* in, float* out) {
+  if (!b || !b->created || !in || !out) return fail(HB2_ERR_ARG, "bad argument");
+  CK(cudaSetDevice(b->P->device));
+  BD& B = b->B;
+  cudaStream_t st = b->stream;
+  const int nc = B.nc;
+  const size_t n = (size_t)B.n, npad = (size_t)B.npad;
+  std::vector<float> xi(npad * nc, 0.f);
+  B.only_cand = -1;
+  if (!adjoint) {
+    for (int c = 0; c < nc; ++c)
+      for (int z = 0; z < B.L3; ++z)
+        for (int pp = 0; pp < B.ndisk; ++pp)
+          xi[c * npad + (size_t)pp * B.L3P + z] = in[c * n + (size_t)z * B.ndisk + b->P->int2ref[pp]];
+    CK(cudaMemcpyAsync(B.xs, xi.data(), sizeof(float) * xi.size(), cudaMemcpyHostToDevice, st));
+    CK(cudaMemsetAsync(B.u, 0, sizeof(float) * (size_t)b->u_total, st));
+    launch_fwd_data(b, MODE_PLAIN);
+    launch_fwd_sym(b, MODE_PLAIN);
+    CKL();
+    long long off = 0;
+    for (int c = 0; c < nc; ++c) {
+      const long long m = (long long)b->h_mdata[c] + b->h_msym[c];
+      CK(cudaMemcpyAsync(out + off, B.u + b->h_uoff[c], sizeof(float) * m, cudaMemcpyDeviceToHost, st));
+      off += m;
+    }
+    CK(cudaStreamSynchronize(st));
+  } else {
+    long long off = 0;
+    for (int c = 0; c < nc; ++c) {
+      const long long m = (long long)b->h_mdata[c] + b->h_msym[c];
+      CK(cudaMemcpyAsync(B.u + b->h_uoff[c], in + off, sizeof(float) * m, cudaMemcpyHostToDevice, st));
+      off += m;
+    }
+    launch_adj(b, MODE_PLAIN);
+    CKL();
+    CK(cudaMemcpyAsync(xi.data(), B.xs, sizeof(float) * xi.size(), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    for (int c = 0; c < nc; ++c)
+      for (int z = 0; z < B.L3; ++z)
+        for (int pp = 0; pp < B.ndisk; ++pp)
+          out[c * n + (size_t)z * B.ndisk + b->P->int2ref[pp]] = xi[c * npad + (size_t)pp * B.L3P + z];
+  }
+  b->solved = false;
+  return HB2_OK;
+}
+
+extern "C" int hb2_batch_solve_model(hb2_batch* b, const hb2_model_options* o, hb2_result* res) {
+  if (!b || !b->created || !o || !res || !o->power_start) return fail(HB2_ERR_ARG, "bad argument");
+  if (o->kind != HB2_MODEL_ENET && o->kind != HB2_MODEL_RIDGE) return fail(HB2_ERR_ARG, "unknown model kind");
+  if (!(o->alpha > 0) || !(o->l1_ratio >= 0 && o->l1_ratio <= 1) || !(o->gap_factor > 0))
+    return fail(HB2_ERR_ARG, "model: alpha > 0, 0 <= l1_ratio <= 1 and gap_factor > 0 are required");
+  if (b->explicit_rows || b->bilinear)
+    return fail(HB2_ERR_GEOMETRY, "model solves run on nearest-neighbour batches only (explicit and trilinear rows: not implemented)");
+  BD& B = b->B;
+  const int nc = B.nc;
+  for (int c = 0; c < nc; ++c)
+    if (b->real_set.empty() || !b->real_set[c]) return fail(HB2_ERR_STATE, "hb2_batch_set_real_rows missing for a candidate");
+  CK(cudaSetDevice(b->P->device));
+  NvtxRange nvtx_("solve_model (batch)");
+  cudaStream_t st = b->stream;
+  const int max_iter = o->max_iter > 0 ? o->max_iter : 4000;
+  const int check = o->check_every > 0 ? o->check_every : 10;
+  const bool enet = o->kind == HB2_MODEL_ENET;
+  B.only_cand = -1;
+  B.clip_pred = o->clip_pred;
+  b->profiling = false;
+  cudaEvent_t e0, e1, e2;
+  CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1)); CK(cudaEventCreate(&e2));
+  CK(cudaEventRecord(e0, st));
+  DevPool tmp;  // scratch from the batch's arena, like run_trf's
+  tmp.owner = b;
+#define CKM(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { tmp.free_all(); return fail(HB2_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_)); } } while (0)
+  MD M{};
+  const size_t nv = (size_t)nc * B.npad;
+  long long max_m = 0;
+  for (int c = 0; c < nc; ++c) max_m = std::max<long long>(max_m, (long long)b->h_mdata[c] + b->h_msym[c]);
+  M.gn = (int)cdiv(B.npad, MDL_SPAN);
+  M.gm = (int)std::max(1u, cdiv(max_m, MDL_SPAN));
+  M.slots = std::max(M.gn, M.gm);
+  M.max_iter = max_iter;
+  M.gap_factor = o->gap_factor;
+  M.real = b->d_real;
+  CKM(tmp.alloc(&M.xbar, nv, true, st));
+  CKM(tmp.alloc(&M.wn, nv, true, st));
+  if (!enet) {
+    CKM(tmp.alloc(&M.rhs, nv, true, st));
+    CKM(tmp.alloc(&M.r, nv, true, st));
+  }
+  double* v0 = nullptr;
+  CKM(tmp.alloc(&v0, (size_t)B.npad, true, st));
+  M.v0 = v0;
+  CKM(tmp.alloc(&M.red, (size_t)nc * M.slots * TRF_NRED, true, st));
+  CKM(tmp.alloc(&M.st, nc, true, st));
+  bool any_fista = false;
+  {
+    std::vector<double> vi((size_t)B.npad, 0.0);  // reference order z*ndisk + p -> internal p*L3P + z
+    for (int z = 0; z < B.L3; ++z)
+      for (int pp = 0; pp < B.ndisk; ++pp) vi[(size_t)pp * B.L3P + z] = o->power_start[(size_t)z * B.ndisk + b->P->int2ref[pp]];
+    std::vector<ModelState> hs(nc);
+    for (int c = 0; c < nc; ++c) {
+      ModelState& S = hs[c];
+      memset(&S, 0, sizeof(S));
+      S.positive = b->cands[c].positive ? 1 : 0;
+      S.kind = enet ? MDL_FISTA_ENET : (S.positive ? MDL_FISTA_RIDGE : MDL_CG_RIDGE);
+      any_fista = any_fista || S.kind != MDL_CG_RIDGE;
+      S.alpha = o->alpha;
+      S.l1_ratio = enet ? o->l1_ratio : 0.0;
+      S.in_power = 1; S.active = 1; S.t = 1.0;
+    }
+    CKM(cudaMemcpyAsync(v0, vi.data(), sizeof(double) * vi.size(), cudaMemcpyHostToDevice, st));
+    CKM(cudaMemcpyAsync(M.st, hs.data(), sizeof(ModelState) * nc, cudaMemcpyHostToDevice, st));
+    CKM(cudaStreamSynchronize(st));  // the host vectors go out of scope
+  }
+  long long launches = 0;
+  b->extra_launches = 0;
+  auto npass = [&](auto op) {
+    constexpr int OP = decltype(op)::value;
+    k_mdl_n<OP><<<dim3(M.gn, nc), HB2_BLOCK, 0, st>>>(B, M);
+    ++launches;
+  };
+  auto mpass = [&](auto op) {
+    constexpr int OP = decltype(op)::value;
+    k_mdl_m<OP><<<dim3(M.gm, nc), HB2_BLOCK, 0, st>>>(B, M);
+    ++launches;
+  };
+  // red(pass, decision, it): combine the partials of the pass just run (its activity gates the decision)
+  auto red = [&](auto op, int sc, int it) {
+    constexpr int OP = decltype(op)::value;
+    k_mdl_reduce<<<nc, HB2_BLOCK, 0, st>>>(M, OP < MM_SETUP ? M.gn : M.gm, mdl_mask(OP), sc, it, OP);
+    ++launches;
+  };
+  // X and X^T over all candidates with the MODE_PLAIN projector kernels (only_cand = -1).  The forward writes only the
+  // rows that exist (rays with data, used column slots: k_fwd_data / k_fwd_tie / k_fwd_band), and a duplicate (Halton)
+  // view's rows are copies written by its first view; so u is zeroed first, as hb2_batch_apply_forward does, and the
+  // row passes read every real row of a defined value.  The forward reads its input from B.xs, the adjoint writes its
+  // output there (n-space passes load / read B.xs around each product).  Tie views and duplicates take their separate
+  // kernels inside launch_fwd_data / launch_adj: MODE_PLAIN keeps dedupe_adj off.
+  auto fwd = [&]() -> cudaError_t {
+    cudaError_t e = cudaMemsetAsync(B.u, 0, sizeof(float) * (size_t)b->u_total, st);
+    launch_fwd_data(b, MODE_PLAIN);
+    launch_fwd_sym(b, MODE_PLAIN);
+    launches += 2;
+    return e;
+  };
+  auto adj = [&]() { launch_adj(b, MODE_PLAIN); ++launches; };
+  using std::integral_constant;
+#define OPM(X) integral_constant<int, X>{}
+  CKM(cudaMemsetAsync(B.x, 0, nv * sizeof(double), st));
+  CKM(cudaMemsetAsync(B.hbar, 0, nv * sizeof(double), st));
+  // m, ybar, ||y_c||^2, xbar = A^T mask / m
+  mpass(OPM(MM_SETUP)); red(OPM(MM_SETUP), MS_SETUP, 0);
+  mpass(OPM(MM_YY)); red(OPM(MM_YY), MS_YY, 0);
+  mpass(OPM(MM_MASK)); adj(); npass(OPM(MN_XBAR));
+  // Lipschitz constant of X_c^T X_c: 20 power steps (skipped when every candidate runs CG)
+  if (any_fista) {
+    npass(OPM(MN_V0));
+    for (int k = 0; k < 20; ++k) {
+      npass(OPM(MN_LOADZ)); red(OPM(MN_LOADZ), MS_S, 0);
+      CKM(fwd()); mpass(OPM(MM_ROW)); red(OPM(MM_ROW), MS_SR, 0);
+      adj(); npass(OPM(MN_POW)); red(OPM(MN_POW), MS_POW, 0);
+      npass(OPM(MN_POWNORM));
+    }
+  }
+  k_mdl_reduce<<<nc, HB2_BLOCK, 0, st>>>(M, 0, 0u, MS_LIP, 0, -1);
+  npass(OPM(MN_ZERO));
+  if (!enet) {  // rhs = X_c^T y_c
+    mpass(OPM(MM_YC)); red(OPM(MM_YC), MS_SR, 0);
+    adj(); npass(OPM(MN_RHS)); red(OPM(MN_RHS), MS_RHS, 0);
+  }
+  CKM(cudaGetLastError());
+  int g = 0, nact = nc;
+  // every refit of a candidate restarts at most max_iter + 9 iterations later; MDL_MAX_REFITS bounds their number
+  const long long g_limit = (long long)(max_iter + 10) * (MDL_MAX_REFITS + 1);
+  while (nact > 0 && g < g_limit) {
+    for (int q = 0; q < check; ++q) {
+      ++g;
+      k_mdl_reduce<<<nc, HB2_BLOCK, 0, st>>>(M, 0, 0u, MS_BEGIN, g, -1);
+      npass(OPM(MN_LOADZ)); red(OPM(MN_LOADZ), MS_S, g);
+      CKM(fwd()); mpass(OPM(MM_ROW)); red(OPM(MM_ROW), MS_SR, g);
+      adj();
+      npass(OPM(MN_GRAD)); red(OPM(MN_GRAD), MS_GRAD, g);
+      npass(OPM(MN_UPD)); red(OPM(MN_UPD), MS_UPD, g);
+      if (!enet) npass(OPM(MN_CGP));
+      if (enet && g % 10 == 0) {  // duality gap of the candidates at their 10th, 20th, ... iteration
+        npass(OPM(MN_LOADW)); red(OPM(MN_LOADW), MS_S, g);
+        CKM(fwd()); mpass(OPM(MM_GAPROW)); red(OPM(MM_GAPROW), MS_GAP, g);
+        adj(); npass(OPM(MN_GAP)); red(OPM(MN_GAP), MS_GAP, g);
+      }
+      launches += 2;
+    }
+    CKM(cudaGetLastError());
+    k_mdl_count<<<1, HB2_BLOCK, 0, st>>>(M.st, nc, b->d_nactive);
+    CKM(cudaMemcpyAsync(b->h_nactive, b->d_nactive, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CKM(cudaStreamSynchronize(st));
+    nact = *b->h_nactive;
+  }
+  CKM(cudaEventRecord(e1, st));
+  // score: float32 w reprojected (launch_fwd_data MODE_SCORE + k_scal_score, as hb2_batch_solve)
+  npass(OPM(MN_FINAL));
+  launch_fwd_data(b, MODE_SCORE);
+  k_scal_score<<<nc, HB2_BLOCK, 0, st>>>(B, b->d_score);
+  k_mdl_publish<<<cdiv(nc, HB2_BLOCK), HB2_BLOCK, 0, st>>>(B, M.st);
+  launches += 3;
+#undef OPM
+  CKM(cudaGetLastError());
+  CKM(cudaEventRecord(e2, st));
+  std::vector<ModelState> hs(nc);
+  std::vector<float> sc(nc);
+  CKM(cudaMemcpyAsync(hs.data(), M.st, sizeof(ModelState) * nc, cudaMemcpyDeviceToHost, st));
+  CKM(cudaMemcpyAsync(sc.data(), b->d_score, sizeof(float) * nc, cudaMemcpyDeviceToHost, st));
+  CKM(cudaStreamSynchronize(st));
+  tmp.free_all();
+#undef CKM
+  float ms_m = 0, ms_s = 0;
+  cudaEventElapsedTime(&ms_m, e0, e1); cudaEventElapsedTime(&ms_s, e1, e2);
+  cudaEventDestroy(e0); cudaEventDestroy(e1); cudaEventDestroy(e2);
+  for (double& t : b->timing) t = 0;
+  b->timing[0] = ms_m; b->timing[2] = ms_s; b->timing[3] = (double)(launches + b->extra_launches); b->timing[4] = g;
+  b->mdl_info.assign((size_t)nc * 4, 0.0);
+  for (int c = 0; c < nc; ++c) {
+    const ModelState& S = hs[c];
+    hb2_result& r = res[c];
+    memset(&r, 0, sizeof(r));
+    r.score = sc[c]; r.itn = S.it;
+    // a candidate still unfinished at g_limit (a right-hand side without signal) counts as not converged
+    r.flags = b->cand_flags[c] | ((S.not_conv || !S.stop) ? HB2_FLAG_NOT_CONVERGED : 0u);
+    r.n_sym_rows = b->h_msym[c];
+    double* inf = &b->mdl_info[(size_t)c * 4];
+    inf[0] = S.alpha; inf[1] = S.it; inf[2] = S.gap; inf[3] = S.kind == MDL_CG_RIDGE ? 0.0 : S.L;
+  }
+  b->last_trf.assign(nc, TrfState{});
+  b->solved = true;
+  return HB2_OK;
+}
+
+extern "C" int hb2_batch_model_info(hb2_batch* b, int32_t c, double* out4) {
+  if (!b || !out4 || c < 0 || (size_t)c * 4 + 4 > b->mdl_info.size()) return fail(HB2_ERR_ARG, "bad argument or no model solve yet");
+  memcpy(out4, &b->mdl_info[(size_t)c * 4], 4 * sizeof(double));
   return HB2_OK;
 }
 

@@ -76,10 +76,25 @@ def main(argv=None):
     ap.add_argument("--batch-candidates", type=int, default=0, help="candidates per batch (default: sized from GPU memory)")
     ap.add_argument("--resume", action="store_true", help="keep the score tiles of solved batches in <output>_img<i>.tiles"
                     "[.rank<r>].npz and restart an interrupted search from them (same image, grid and parameters)")
+    ap.add_argument("--model", default="lsq", choices=["lsq", "elasticnet", "lasso", "ridge"],
+                    help="solver model (app.py algorithm; default lsq)")
+    ap.add_argument("--alpha", type=float, default=None, help="model alpha (default: 1 for ridge, 1e-4 otherwise)")
+    ap.add_argument("--l1-ratio", type=float, default=None, help="elastic-net l1_ratio (default 0.5)")
     args = ap.parse_args(argv)
+    algorithm = None
+    if args.model != "lsq":
+        algorithm = dict(model=args.model)
+        if args.alpha is not None:
+            algorithm["alpha"] = args.alpha
+        if args.l1_ratio is not None:
+            algorithm["l1_ratio"] = args.l1_ratio
+    elif args.alpha is not None or args.l1_ratio is not None:
+        ap.error("--alpha / --l1-ratio need --model elasticnet, lasso or ridge")
 
     from . import distributed, pipeline, transforms
-    from .grid import search_grid
+    from .grid import check_algorithm, search_grid
+
+    check_algorithm(algorithm, args.interpolation)  # before any GPU work
 
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -110,7 +125,7 @@ def main(argv=None):
                           positive_constraint=args.positive_constraint, top_k=args.top_k, device=local_rank,
                           shard=(rank, world), return_x_top=args.save_map, interpolation=args.interpolation, dist=dist,
                           checkpoint=f"{args.output}_img{i}.tiles" if args.resume else None,
-                          batch_candidates=args.batch_candidates or None)
+                          batch_candidates=args.batch_candidates or None, algorithm=algorithm)
         # with more than one process the per-rank score maps were all-gathered inside search_grid (one NCCL call)
         if rank != 0:
             continue
@@ -139,7 +154,8 @@ def main(argv=None):
                 positive_constraint=args.positive_constraint, reconstruct_diameter_3d_inner_pixel=g["D3i"],
                 reconstruct_diameter_2d_pixel=g["D2"], reconstruct_length_2d_pixel=g["L2"],
                 reconstruct_diameter_3d_pixel=g["D3"], reconstruct_length_3d_pixel=g["L3"],
-                sym_oversample=g["sym_oversample"], interpolation=args.interpolation, device=local_rank)
+                sym_oversample=g["sym_oversample"], interpolation=args.interpolation, device=local_rank,
+                algorithm=algorithm or dict(model="lsq"))
         if args.save_map and best is not None and "rec3d" in best:
             ny, nx = img.shape
             vol = transforms.apply_helical_symmetry(best["rec3d"], apix, best["twist"], best["rise"], csym=best["csym"],

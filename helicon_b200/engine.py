@@ -17,6 +17,26 @@ DEFAULT_OPTIONS = dict(
 )
 
 
+MODELS = ("elasticnet", "lasso", "ridge")
+
+
+def model_params(algorithm):
+    """(kind, alpha, l1_ratio) of a sklearn-model ``algorithm`` dict with the reference's defaults (alpha 1 for ridge,
+    1e-4 otherwise; l1_ratio 0.5), or None for ``None`` / ``{"model": "lsq"}``.  Raises before any GPU work."""
+    model = "lsq" if algorithm is None else algorithm.get("model", "lsq")
+    if model == "lsq":
+        return None
+    if model not in MODELS:
+        raise NotImplementedError(f"helicon_b200: algorithm model {model!r} is not implemented on the CUDA path "
+                                  "(lsq, elasticnet, lasso, ridge are; 'lreg' / 'ard' need the dense matrix)")
+    alpha = float(algorithm.get("alpha", 1 if model == "ridge" else 1e-4))
+    l1_ratio = 1.0 if model == "lasso" else (0.0 if model == "ridge" else float(algorithm.get("l1_ratio", 0.5)))
+    if not alpha > 0 or not 0 <= l1_ratio <= 1:
+        raise ValueError(f"helicon_b200: model {model!r} needs alpha > 0 and 0 <= l1_ratio <= 1 "
+                         f"(got alpha={alpha}, l1_ratio={l1_ratio})")
+    return model, alpha, l1_ratio
+
+
 def _stream_handle(stream):
     if stream is None:
         return None
@@ -207,6 +227,61 @@ class Batch:
         res["n_data_rows"] = self.plan.cand_n_data_rows
         self.results = res
         return res
+
+    def real_rows(self, c):
+        """Mask of the real rows of candidate ``c`` over its padded rows (data rows of ``data_row_index`` and every
+        symmetry row), as regularized._CenteredOperator builds it."""
+        nd_pad, tot = self.rows_padded(c)
+        real = np.zeros(tot, dtype=np.uint8)
+        real[self.data_row_index(c)[0]] = 1
+        real[nd_pad:] = 1
+        return real
+
+    def solve_model(self, algorithm, clip_pred=0, gap_factor=0.05, max_iter=4000, check_every=10):
+        """ElasticNet / Lasso / Ridge (SLR:272-342) for every candidate at once on the device (hb2_batch_solve_model):
+        the objectives, schedule and stop rules of regularized.solve_model; each candidate's positive constraint is its
+        CandidateSpec.positive.  Returns the result array of ``solve`` (itn = iterations of the final fit, flags with
+        HB2_FLAG_NOT_CONVERGED where max_iter ended it)."""
+        model, alpha, l1_ratio = model_params(algorithm)
+        lib = _lib.load()
+        if not getattr(self, "_real_set", False):
+            for c in range(self.nc):
+                real = self.real_rows(c)
+                _lib.check(lib.hb2_batch_set_real_rows(self._h, c, _lib.ptr(real), len(real)))
+            self._real_set = True
+        v = np.random.default_rng(0).standard_normal(self.n)
+        v /= np.linalg.norm(v)
+        o = _lib.ModelOptions(kind=_lib.MODEL_RIDGE if model == "ridge" else _lib.MODEL_ENET, alpha=alpha,
+                              l1_ratio=l1_ratio, gap_factor=float(gap_factor), max_iter=int(max_iter),
+                              check_every=int(check_every), clip_pred=int(clip_pred), power_start=_lib.ptr(v))
+        res = np.zeros(self.nc, dtype=_lib.RESULT_DTYPE)
+        _lib.check(lib.hb2_batch_solve_model(self._h, C.byref(o), _lib.ptr(res)))
+        res["n_data_rows"] = self.plan.cand_n_data_rows
+        self.results = res
+        return res
+
+    def model_info(self, c):
+        """dict(alpha, iterations, gap, lipschitz) of candidate ``c``'s final fit (gap: the relative CG residual for
+        ridge, the last relative update for ridge with the positive constraint; lipschitz 0 for CG)."""
+        out = np.zeros(4, dtype=np.float64)
+        _lib.check(_lib.load().hb2_batch_model_info(self._h, int(c), _lib.ptr(out)))
+        return dict(alpha=float(out[0]), iterations=int(out[1]), gap=float(out[2]), lipschitz=float(out[3]))
+
+    def apply_all(self, xs=None, ys=None):
+        """The MODE_PLAIN products over all candidates in one launch each (tests): ``xs`` [nc, n] -> list of row
+        vectors, or ``ys`` (list of row vectors) -> [nc, n]."""
+        lib = _lib.load()
+        tots = [self.rows_padded(c)[1] for c in range(self.nc)]
+        if xs is not None:
+            x = np.ascontiguousarray(xs, dtype=np.float32).reshape(self.nc, self.n)
+            y = np.empty(sum(tots), dtype=np.float32)
+            _lib.check(lib.hb2_batch_apply_all(self._h, 0, _lib.ptr(x), _lib.ptr(y)))
+            return np.split(y, np.cumsum(tots)[:-1])
+        y = np.ascontiguousarray(np.concatenate([np.asarray(v, dtype=np.float32) for v in ys]))
+        assert len(y) == sum(tots)
+        x = np.empty((self.nc, self.n), dtype=np.float32)
+        _lib.check(lib.hb2_batch_apply_all(self._h, 1, _lib.ptr(y), _lib.ptr(x)))
+        return x
 
     def timing(self):
         out = np.zeros(16, dtype=np.float64)

@@ -17,7 +17,7 @@ from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
 
-from .engine import Batch, ExplicitBatch, Problem, ScoreMap, Stream
+from .engine import Batch, ExplicitBatch, Problem, ScoreMap, Stream, model_params
 from .planner import MAX_EQUATIONS, CandidateSpec, positive_rule
 
 logger = logging.getLogger(__name__)
@@ -246,12 +246,24 @@ def build_tasks(ny, nx, apix, twists, rises, csyms=(1,), reconstruct_length_rise
     return tasks, ti
 
 
-def _bytes_per_candidate(n, md, cap):
-    return 8 * (md + cap) + 48 * n + 16 * cap + 8 * cap + 32 * (2 * cap + 17) + 16 * n + 12 * (n + 1)
+def _bytes_per_candidate(n, md, cap, model=False):
+    """Device bytes of one candidate; ``model``: hb2_batch_solve_model adds xbar, w_new, rhs and the CG residual
+    (float64 n-vectors) and the one-byte real-row mask."""
+    extra = 32 * n + (md + cap) if model else 0
+    return 8 * (md + cap) + 48 * n + 16 * cap + 8 * cap + 32 * (2 * cap + 17) + 16 * n + 12 * (n + 1) + extra
+
+
+def check_algorithm(algorithm, interpolation="nn"):
+    """model_params of ``algorithm``, refusing what the batched model path does not cover (before any GPU work)."""
+    params = model_params(algorithm)
+    if params is not None and interpolation != "nn":
+        raise NotImplementedError("helicon_b200: a grid search with a sklearn model runs on nearest-neighbour batches "
+                                  "only (interpolation='linear' with a model is not implemented)")
+    return params
 
 
 def make_chunks(tasks, ndisk_of, batch_candidates=None, mem_budget_bytes=48 << 30, pipelined=True, positive_constraint=-1,
-                interpolation="nn"):
+                interpolation="nn", model=False):
     """Cut the (twist-major) task list into the chunks that are solved as one batch each, most expensive first.
 
     Tasks that share a Problem/Batch shape (D2, L2, D3, D3i, s, L3) are grouped; every group is cut into runs of
@@ -273,7 +285,7 @@ def make_chunks(tasks, ndisk_of, batch_candidates=None, mem_budget_bytes=48 << 3
                                    positive_rule(positive_constraint, rise_px, t.twist, L3))
         md_est = int((L3 + L2) / max(min(x.spec.rise_pixel for x in tl), 1e-3) + 3) * L3 * D2
         cap_est = min(max(x.spec.min_sym_pairs for x in tl) + n3, 64 * n3)
-        per_cand = _bytes_per_candidate(n3, md_est, cap_est) * (2 if pipelined else 1)  # two batches resident
+        per_cand = _bytes_per_candidate(n3, md_est, cap_est, model) * (2 if pipelined else 1)  # two batches resident
         bs = batch_candidates or max(1, min(512, int(mem_budget_bytes // per_cand)))
         if interpolation != "nn":
             # trilinear rows: matrix-free batches where the factorisation applies (bilinear.py; ~0.3 GB per candidate:
@@ -291,7 +303,7 @@ def search_grid(image, apix, twists, rises, csyms=(1,), reconstruct_length_rise=
                 tube_diameter_inner=0.0, tube_length=None, target_apix3d=0, sym_oversample=-1,
                 positive_constraint=-1, thresh_fraction=-1, top_k=10, device=0, stream=None, batch_candidates=None,
                 mem_budget_bytes=48 << 30, shard=(0, 1), return_x_top=False, progress=None, pipelined=True,
-                interpolation="nn", dist=None, checkpoint=None, checkpoint_seconds=30.0):
+                interpolation="nn", dist=None, checkpoint=None, checkpoint_seconds=30.0, algorithm=None):
     """Solve + score every candidate of the grid on one GPU (or this rank's share of it).
 
     ``interpolation="nn"`` runs batches of candidates through the matrix-free projector; ``"linear"`` (trilinear rows,
@@ -309,9 +321,14 @@ def search_grid(image, apix, twists, rises, csyms=(1,), reconstruct_length_rise=
     batches are written to ``path`` (``path.rank<r>`` per rank) every ``checkpoint_seconds``; a later call with the same
     image, grid and parameters restores them into the device maps (``hb2_scoremap_restore``) and solves only the rest
     (``n_restored`` in the result; ``return_x_top`` volumes exist only for candidates solved in this call).
+    ``algorithm`` (the app's solver choice, SLR:272-342): None or ``{"model": "lsq"}`` runs LSMR (+ the bounded branch);
+    ``{"model": "elasticnet" | "lasso" | "ridge", "alpha": .., "l1_ratio": ..}`` the batched model solver
+    (Batch.solve_model) with the reference's defaults; other models and ``interpolation="linear"`` with a model raise
+    NotImplementedError before any GPU work.
     Returns dict(scores[(n_csym,) T, R] (NaN = not solved here / skipped task), itn, flags, top,
     n_candidates, seconds).
     """
+    mparams = check_algorithm(algorithm, interpolation)
     ny, nx = np.asarray(image).shape
     tube_d = ny * apix if tube_diameter is None else tube_diameter
     image = prepare_image(image, thresh_fraction, tube_d if 0 < tube_d < ny * apix else ny * apix, apix)
@@ -332,7 +349,8 @@ def search_grid(image, apix, twists, rises, csyms=(1,), reconstruct_length_rise=
                          reconstruct_length_rise=reconstruct_length_rise, tube_diameter=tube_diameter,
                          tube_diameter_inner=tube_diameter_inner, tube_length=tube_length, target_apix3d=target_apix3d,
                          sym_oversample=sym_oversample, positive_constraint=positive_constraint,
-                         clip_pred=int(thresh_fraction >= 0), interpolation=str(interpolation), library=_version())
+                         clip_pred=int(thresh_fraction >= 0), interpolation=str(interpolation), library=_version(),
+                         **model_fingerprint(mparams))
         store = ScoreTileStore(checkpoint, fp, ntot, rank=rank, world=world, flush_seconds=checkpoint_seconds)
         if world > 1 and dist is not None and dist.is_available() and dist.is_initialized():
             agree_across_ranks(store, dist, device)  # every rank must filter the SAME tasks
@@ -348,7 +366,7 @@ def search_grid(image, apix, twists, rises, csyms=(1,), reconstruct_length_rise=
         return probs[key]
 
     chunks = make_chunks(tasks, lambda key: problem(key).ndisk, batch_candidates, mem_budget_bytes, pipelined,
-                         positive_constraint, interpolation)
+                         positive_constraint, interpolation, model=mparams is not None)
     queue = ChunkQueue(len(chunks), shard=shard, dist=dist)
     smap = ScoreMap(ntot, device=device)  # score / iteration / flag maps + top-K live on the device
     top_x = {}
@@ -373,7 +391,7 @@ def search_grid(image, apix, twists, rises, csyms=(1,), reconstruct_length_rise=
 
     try:
         stats = solve_chunks(chunks, queue, problem, device=device, pipelined=pipelined, interpolation=interpolation,
-                             clip_pred=int(thresh_fraction >= 0), on_result=on_result)
+                             clip_pred=int(thresh_fraction >= 0), on_result=on_result, algorithm=algorithm if mparams else None)
         n_solved = stats["n_candidates"]
         if dist is not None and dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
             # the ONLY collective of a search: every rank's maps all-gathered (NCCL), folded and ranked on the device
@@ -419,13 +437,22 @@ TIMING_KEYS = ("lsmr_ms", "trf_ms", "score_ms", "fwd_data_ms", "fwd_sym_ms", "ad
                "launches", "fwd_data_launches", "adj_launches", "update_launches")
 
 
+def model_fingerprint(mparams):
+    """Checkpoint parameters of the solver model: none for lsq, so that the tiles of existing lsq searches resume."""
+    if mparams is None:
+        return {}
+    model, alpha, l1_ratio = mparams
+    return dict(model=model, alpha=float(alpha), l1_ratio=float(l1_ratio))
+
+
 def solve_chunks(chunks, queue, problem_of, device=0, pipelined=True, interpolation="nn", clip_pred=0, profile=0,
-                 on_result=None, solve_options=None):
+                 on_result=None, solve_options=None, algorithm=None):
     """Solve the chunks ``queue`` deals to this rank: ``chunks[i] = (problem key, [GridTask], cost)`` (make_chunks).
 
     The batch of chunk i+1 is planned and set up by a worker thread (second stream) while chunk i is being solved
     (BatchPipeline).  ``on_result(chunk_tasks, results, batch)`` is called per solved batch, before it is closed.
-    Returns the summed library timings (``profile=1`` adds the per-kernel-class device times)."""
+    Returns the summed library timings (``profile=1`` adds the per-kernel-class device times).  ``algorithm``: a
+    sklearn-model dict solves every batch with Batch.solve_model instead of LSMR."""
     pipe = BatchPipeline(device=device, pipelined=pipelined)
     stats = dict.fromkeys(TIMING_KEYS, 0.0)
     stats.update(n_candidates=0, n_chunks=0, itn_sum=0, chunk_ids=[])
@@ -448,7 +475,10 @@ def solve_chunks(chunks, queue, problem_of, device=0, pipelined=True, interpolat
         for ci, batch in batches:
             chunk = chunks[ci][1]
             try:
-                res = batch.solve(clip_pred=clip_pred, profile=int(profile), **opts)
+                if algorithm is not None:
+                    res = batch.solve_model(algorithm, clip_pred=clip_pred, **opts)
+                else:
+                    res = batch.solve(clip_pred=clip_pred, profile=int(profile), **opts)
                 tm = batch.timing()
                 for k in TIMING_KEYS:
                     stats[k] += tm.get(k, 0.0)

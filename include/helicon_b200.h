@@ -40,6 +40,7 @@ typedef enum {
 #define HB2_FLAG_BOUNDED 4u      /* the bounded (TRF) branch ran (SLR:246-270, scipy lsq_linear) */
 #define HB2_FLAG_NO_ROWS 8u      /* no data rows */
 #define HB2_FLAG_TIE_Z_EXACT 16u /* column->slice ties resolved per sample from the reference's z table (exact) */
+#define HB2_FLAG_NOT_CONVERGED 32u /* hb2_batch_solve_model: max_iter ended the fit before its stop rule held */
 
 typedef struct hb2_problem hb2_problem; /* one image + in-plane geometry, shared by many candidates */
 typedef struct hb2_batch hb2_batch;     /* a set of candidates solved together */
@@ -309,6 +310,41 @@ int hb2_batch_timing(hb2_batch* b, double* out16);
  * cost, g_norm, inner LSMR iterations, step kind (0 full Newton, 1 truncated Newton, 2 reflected, 3 anti-gradient),
  * p_value, r_value, ag_value, cost_change.  Returns nit*16 + (status+1). */
 int hb2_batch_trf_trace(hb2_batch* b, int32_t cand, double* out, int32_t max_rows);
+
+/* ---- ElasticNet / Lasso / Ridge (SLR:272-342) for every candidate of a nearest-neighbour batch ---------------
+ * The reference's scikit-learn models on the stacked system [A_data; A_hsym] x = [b; 0] with the intercept profiled
+ * out (X and y centred over the candidate's REAL rows), minimised as helicon_b200/regularized.py does on the host:
+ * FISTA with adaptive restart and scikit-learn's duality gap for elastic net / lasso (and for ridge with the positive
+ * constraint), CG on the normal equations for ridge, and the refit of an all-zero solution with alpha x 0.1
+ * (SLR:331-335).  All candidates run at once on the device; the host only polls a counter every check_every iterations.
+ * The positive constraint of each candidate is hb2_candidate.positive.  Afterwards the batch is solved as after
+ * hb2_batch_solve: hb2_batch_get_x, hb2_batch_scatter_scores and the score (float32 w reprojected) are the model's,
+ * hb2_result.itn = iterations of the final fit, flags |= HB2_FLAG_NOT_CONVERGED where max_iter ended it. */
+#define HB2_MODEL_ENET 0   /* elastic net; lasso is l1_ratio = 1 */
+#define HB2_MODEL_RIDGE 1
+typedef struct {
+  int32_t kind;               /* HB2_MODEL_ENET or HB2_MODEL_RIDGE */
+  double alpha;               /* > 0 (scikit-learn's alpha) */
+  double l1_ratio;            /* [0, 1], elastic net only */
+  double gap_factor;          /* stop at gap <= gap_factor * 1e-2 * ||y_c||^2 (0.05: 20x tighter than the reference) */
+  int32_t max_iter;           /* iterations per fit (4000) */
+  int32_t check_every;        /* host polls the active-candidate counter every this many iterations */
+  int32_t clip_pred;          /* as hb2_solve_options.clip_pred */
+  const double* power_start;  /* [n] start vector of the power iteration for the Lipschitz constant, reference order,
+                                 unit norm (regularized.py: default_rng(0).standard_normal(n) normalised) */
+} hb2_model_options;
+/* The candidate's real rows: real[m] over its padded row space (data rows then symmetry rows, m = the total of
+ * hb2_batch_rows_padded), 1 where the row is an equation of the reference's system (Batch.data_row_index and every
+ * symmetry row).  Required for every candidate before hb2_batch_solve_model. */
+int hb2_batch_set_real_rows(hb2_batch* b, int32_t cand, const uint8_t* real, int64_t m);
+int hb2_batch_solve_model(hb2_batch* b, const hb2_model_options* opt, hb2_result* results_host);
+/* after hb2_batch_solve_model: out[4] = final alpha, iterations of the final fit, duality gap (elastic net; ridge: the
+ * relative CG residual, or the last relative update with the positive constraint), Lipschitz estimate (0 for CG) */
+int hb2_batch_model_info(hb2_batch* b, int32_t cand, double* out4);
+/* test hook: the MODE_PLAIN products over ALL candidates in one launch each.  adjoint = 0: in = x of every candidate
+ * ([nc][n], reference order), out = rows ([nc][total padded rows of hb2_batch_rows_padded] concatenated); adjoint = 1:
+ * the other way round. */
+int hb2_batch_apply_all(hb2_batch* b, int32_t adjoint, const float* in_host, float* out_host);
 
 /* ---- test hook: the LSMR scalar recurrences run on the HOST --------------- */
 /* Same code as the device path (compiled __host__ __device__).  state64 is an
