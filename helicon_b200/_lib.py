@@ -67,6 +67,9 @@ class ModelOptions(C.Structure):
 
 MODEL_ENET, MODEL_RIDGE = 0, 1
 
+# score_metric names of lsq_reconstruct / search_grid -> HB2_METRIC_* (cosine is the solve's own score)
+METRICS = {"ssim": 1, "ms_ssim": 2, "mutual_information": 3, "composite": 4}
+
 
 class SymmParams(C.Structure):
     _fields_ = [
@@ -117,6 +120,7 @@ EXPORTS = [
     "hb2_scoremap_create", "hb2_scoremap_destroy", "hb2_scoremap_device_ptr", "hb2_batch_scatter_scores",
     "hb2_scoremap_merge", "hb2_scoremap_topk", "hb2_scoremap_read", "hb2_scoremap_restore",
     "hb2_batch_set_real_rows", "hb2_batch_solve_model", "hb2_batch_model_info", "hb2_batch_apply_all",
+    "hb2_batch_set_pixel_rows", "hb2_batch_score_metric",
 ]
 
 _lib = None
@@ -180,6 +184,8 @@ def load():
     lib.hb2_batch_solve_model.argtypes = [vp, P(ModelOptions), vp]
     lib.hb2_batch_model_info.argtypes = [vp, i32, vp]
     lib.hb2_batch_apply_all.argtypes = [vp, i32, vp, vp]
+    lib.hb2_batch_set_pixel_rows.argtypes = [vp, i32, vp, i32, i32]
+    lib.hb2_batch_score_metric.argtypes = [vp, i32, i32, vp, vp]
     lib.hb2_helical_symmetrize.argtypes = [vp, P(SymmParams), vp, vp, vp, vp, vp, vp, i32, vp, vp, vp, vp, C.c_int, vp]
     lib.hb2_lsmr_scalar_step.argtypes = [vp, C.c_int, C.c_float, C.c_float, f64, f64, f64, f64, C.c_int, P(C.c_float), P(C.c_float), P(C.c_float), vp]
     lib.hb2_scoremap_create.argtypes = [P(vp), i64, C.c_int]

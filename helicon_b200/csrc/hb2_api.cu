@@ -9,6 +9,7 @@
 #include "hb2_explicit.cuh"
 #include "hb2_bilinear.cuh"
 #include "hb2_model.cuh"
+#include "hb2_metric.cuh"
 
 #include <cub/cub.cuh>
 #include <nvtx3/nvToolsExt.h>
@@ -293,6 +294,11 @@ struct hb2_batch {
   uint8_t* d_real = nullptr;
   std::vector<uint8_t> real_set;
   std::vector<double> mdl_info;
+  // 2-D score metrics (hb2_batch_score_metric): per-candidate pixel tables [nc][L2*D2]
+  int* d_pixrow = nullptr;
+  std::vector<uint8_t> pixrow_set;
+  float* d_cos = nullptr;   // the solve's cosine scores, kept while d_score holds a metric
+  bool cos_kept = false;    // d_cos holds the scores of the last solve
   std::vector<cudaEvent_t> ev_pool;
   std::vector<std::pair<int, int>> ev_used;  // (class, index of start event)
   size_t ev_next = 0;
@@ -2412,6 +2418,7 @@ extern "C" int hb2_batch_solve(hb2_batch* b, const hb2_solve_options* opt, hb2_r
     r.normr = (float)hs[c].normr; r.normar = hs[c].normar; r.normA = (float)hs[c].normA; r.normx = (float)hs[c].normx;
   }
   b->solved = true;
+  b->cos_kept = false;
   b->last_trf = trf;
   return HB2_OK;
 }
@@ -2665,12 +2672,173 @@ extern "C" int hb2_batch_solve_model(hb2_batch* b, const hb2_model_options* o, h
   }
   b->last_trf.assign(nc, TrfState{});
   b->solved = true;
+  b->cos_kept = false;
   return HB2_OK;
 }
 
 extern "C" int hb2_batch_model_info(hb2_batch* b, int32_t c, double* out4) {
   if (!b || !out4 || c < 0 || (size_t)c * 4 + 4 > b->mdl_info.size()) return fail(HB2_ERR_ARG, "bad argument or no model solve yet");
   memcpy(out4, &b->mdl_info[(size_t)c * 4], 4 * sizeof(double));
+  return HB2_OK;
+}
+
+// ---------------------------------------------------------------------------
+// 2-D score metrics of every candidate (hb2_metric.cuh)
+// ---------------------------------------------------------------------------
+extern "C" int hb2_batch_set_pixel_rows(hb2_batch* b, int32_t c, const int32_t* last_row, int32_t L2, int32_t D2) {
+  if (!b || !b->created || !last_row || c < 0 || c >= b->B.nc) return fail(HB2_ERR_ARG, "bad argument");
+  if (L2 != b->P->g.L2 || D2 != b->P->g.D2) return fail(HB2_ERR_ARG, "pixel table: L2, D2 are not the problem's");
+  const size_t HW = (size_t)L2 * D2;
+  for (size_t p = 0; p < HW; ++p)
+    if (last_row[p] < -1 || last_row[p] >= b->h_mdata[c])
+      return fail(HB2_ERR_ARG, "pixel table: an entry is not -1 or a padded data row of the candidate");
+  CK(cudaSetDevice(b->P->device));
+  if (!b->d_pixrow) {
+    CK(b->pool.alloc(&b->d_pixrow, HW * b->B.nc, false, b->stream));
+    b->pixrow_set.assign(b->B.nc, 0);
+  }
+  CK(cudaMemcpyAsync(b->d_pixrow + HW * c, last_row, sizeof(int32_t) * HW, cudaMemcpyHostToDevice, b->stream));
+  CK(cudaStreamSynchronize(b->stream));  // the host buffer may go away after the call
+  b->pixrow_set[c] = 1;
+  return HB2_OK;
+}
+
+extern "C" int hb2_batch_score_metric(hb2_batch* b, int32_t metric, int32_t clip_pred, float* scores_host, double* parts_host) {
+  if (!b || !b->created) return fail(HB2_ERR_ARG, "bad argument");
+  if (metric < HB2_METRIC_SSIM || metric > HB2_METRIC_COMPOSITE) return fail(HB2_ERR_ARG, "unknown metric");
+  if (!b->solved) return fail(HB2_ERR_STATE, "hb2_batch_score_metric before a solve");
+  BD& B = b->B;
+  const int nc = B.nc;
+  for (int c = 0; c < nc; ++c)
+    if (b->pixrow_set.empty() || !b->pixrow_set[c]) return fail(HB2_ERR_STATE, "hb2_batch_set_pixel_rows missing for a candidate");
+  const hb2_geometry& g = b->P->g;
+  // the reference region image[ny//2 - D2//2 : + D2, nx//2 - L2//2 : + L2] must lie inside the image (numpy slicing)
+  if (g.ny / 2 - g.D2 / 2 < 0 || g.ny / 2 - g.D2 / 2 + g.D2 > g.ny || g.nx / 2 - g.L2 / 2 < 0 || g.nx / 2 - g.L2 / 2 + g.L2 > g.nx)
+    return fail(HB2_ERR_GEOMETRY, "2-D metrics: the (D2, L2) region is not inside the image");
+  CK(cudaSetDevice(b->P->device));
+  NvtxRange nvtx_("score metric (batch)");
+  cudaStream_t st = b->stream;
+  const bool all = parts_host != nullptr;
+  const bool want_ssim = all || metric == HB2_METRIC_SSIM || metric == HB2_METRIC_COMPOSITE;
+  const bool want_ms = all || metric == HB2_METRIC_MS_SSIM || metric == HB2_METRIC_COMPOSITE;
+  const bool want_mi = all || metric == HB2_METRIC_MI || metric == HB2_METRIC_COMPOSITE;
+  // scales of ms_ssim_score: sides round(n / 2) (half to even), computed while both sides are >= 8
+  int Hs[MET_MAX_SCALES], Ws[MET_MAX_SCALES];
+  long long off[MET_MAX_SCALES + 1];
+  int nscale = 1;
+  Hs[0] = g.L2; Ws[0] = g.D2; off[0] = 0;
+  off[1] = (long long)Hs[0] * Ws[0];
+  while (want_ms && nscale < MET_MAX_SCALES && std::min(Hs[nscale - 1], Ws[nscale - 1]) >= 8) {
+    const int h = (int)std::nearbyint(Hs[nscale - 1] * 0.5), w = (int)std::nearbyint(Ws[nscale - 1] * 0.5);
+    if (std::min(h, w) < 8) break;  // ms_ssim_score stops before this scale: its image is never used
+    Hs[nscale] = h; Ws[nscale] = w;
+    off[nscale + 1] = off[nscale] + (long long)h * w;
+    ++nscale;
+  }
+  const long long HW = off[1], stride = off[nscale];
+  if (!b->d_cos) CK(b->pool.alloc(&b->d_cos, (size_t)nc, false, st));  // before the scratch: the arena is a stack
+  cudaEvent_t e0, e1;
+  CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
+  CK(cudaEventRecord(e0, st));
+  DevPool tmp;  // scratch from the batch's arena, like run_trf's
+  tmp.owner = b;
+#define CKS(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { tmp.free_all(); cudaEventDestroy(e0); cudaEventDestroy(e1); return fail(HB2_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_)); } } while (0)
+  double *img = nullptr, *ta = nullptr, *tb = nullptr, *part = nullptr, *parts = nullptr;
+  double2* rng = nullptr;
+  MetCand* ms = nullptr;
+  int* hist = nullptr;
+  const int tx0 = (int)cdiv(std::max(Ws[0] - 6, 1), MET_T), ty0 = (int)cdiv(std::max(Hs[0] - 6, 1), MET_T);
+  CKS(tmp.alloc(&img, (size_t)stride * (nc + 1), false, st));
+  if (nscale > 1) {
+    CKS(tmp.alloc(&ta, (size_t)HW * (nc + 1), false, st));
+    CKS(tmp.alloc(&tb, (size_t)HW * (nc + 1), false, st));
+  }
+  CKS(tmp.alloc(&rng, (size_t)nc + 1, true, st));
+  CKS(tmp.alloc(&ms, (size_t)nc, true, st));
+  CKS(tmp.alloc(&part, (size_t)nc * tx0 * ty0, true, st));
+  if (want_mi) CKS(tmp.alloc(&hist, (size_t)nc * 4096, true, st));
+  if (all) CKS(tmp.alloc(&parts, (size_t)nc * 4, true, st));
+  // the prediction of every candidate: one MODE_PLAIN forward of the batch's float32 x (u zeroed first, as
+  // hb2_batch_apply_forward does), then the last-writer gather
+  B.only_cand = -1;
+  CKS(cudaMemsetAsync(B.u, 0, sizeof(float) * (size_t)b->u_total, st));
+  launch_fwd_data(b, MODE_PLAIN);
+  k_met_gather<<<dim3(cdiv(HW, HB2_BLOCK), nc), HB2_BLOCK, 0, st>>>(B, b->d_pixrow, (int)HW, clip_pred ? 1 : 0, img, stride);
+  k_met_ref<<<cdiv(HW, HB2_BLOCK), HB2_BLOCK, 0, st>>>(b->P->d_pix, Hs[0], Ws[0], img + (size_t)nc * stride);
+  if (!b->cos_kept) {  // later calls after the same solve start from its cosine scores again
+    CKS(cudaMemcpyAsync(b->d_cos, b->d_score, sizeof(float) * nc, cudaMemcpyDeviceToDevice, st));
+    b->cos_kept = true;
+  }
+  std::vector<MetCand> hs(nc);
+  for (auto& S : hs) { memset(&S, 0, sizeof(S)); S.active = 1; }
+  CKS(cudaMemcpyAsync(ms, hs.data(), sizeof(MetCand) * nc, cudaMemcpyHostToDevice, st));
+  k_met_range<<<nc + 1, HB2_BLOCK, 0, st>>>(img, stride, (int)HW, nc, ms, rng);
+  if (want_mi) {
+    k_met_hist<<<dim3(cdiv(HW, MET_HIST_PIX), nc), HB2_BLOCK, 0, st>>>(img, stride, (int)HW, nc, rng, hist);
+    k_met_mi<<<nc, HB2_BLOCK, 0, st>>>(hist, nc, rng, ms);
+  }
+  // Scale 0 of ssim_score / ms_ssim_score: data_range = max(ptp(pred), ptp(ref)) of the float32 images, a float32, so
+  // C1 = (0.01 * R) ** 2 is numpy's float32 power, i.e. libm's powf (called through a pointer that the compiler can
+  // not fold into R * R, which differs from powf in the last bit for some R).
+  if (want_ssim || want_ms) {
+    std::vector<double2> hr(nc + 1);
+    CKS(cudaMemcpyAsync(hr.data(), rng, sizeof(double2) * (nc + 1), cudaMemcpyDeviceToHost, st));
+    CKS(cudaMemcpyAsync(hs.data(), ms, sizeof(MetCand) * nc, cudaMemcpyDeviceToHost, st));
+    CKS(cudaStreamSynchronize(st));
+    static float (*volatile powf_p)(float, float) = powf;
+    const float rr = (float)hr[nc].y - (float)hr[nc].x;
+    for (int c = 0; c < nc; ++c) {
+      const float rp = (float)hr[c].y - (float)hr[c].x;
+      const float R = std::max(rp, rr);
+      hs[c].active = R != 0.f && std::min(Hs[0], Ws[0]) >= 7;  // 0.0 for a zero range and for a side below 7
+      hs[c].c1 = (double)powf_p(0.01f * R, 2.0f);
+      hs[c].c2 = (double)powf_p(0.03f * R, 2.0f);
+    }
+    CKS(cudaMemcpyAsync(ms, hs.data(), sizeof(MetCand) * nc, cudaMemcpyHostToDevice, st));
+    for (int s = 0; s < nscale; ++s) {
+      const int H = Hs[s], W = Ws[s];
+      const int ms_take = want_ms && std::min(H, W) >= 8;
+      if (std::min(H, W) < 7 || (s == 0 && !want_ssim && !ms_take)) break;  // ssim_score: 0.0 below 7
+      const int tx = (int)cdiv(W - 6, MET_T), ty = (int)cdiv(H - 6, MET_T);
+      double* im = img + off[s];
+      k_met_ssim<<<dim3(tx, ty, nc), HB2_BLOCK, 0, st>>>(im, stride, H, W, s, nc, ms, rng, part);
+      k_met_ssim_fin<<<nc, HB2_BLOCK, 0, st>>>(part, tx * ty, (double)(H - 6) * (W - 6), s, ms_take, ms);
+      if (s + 1 >= nscale) break;
+      // _rescale(img, 0.5, order=1) of both images: Gaussian along axis 0, axis 1, then the linear zoom and the clip
+      const int Ho = Hs[s + 1], Wo = Ws[s + 1];
+      MetGauss gy{}, gx{};
+      for (int a = 0; a < 2; ++a) {
+        MetGauss& G = a == 0 ? gy : gx;
+        const double z = a == 0 ? (double)H / Ho : (double)W / Wo;
+        const double sigma = std::max(0.0, (z - 1) / 2);
+        G.r = (int)(4.0 * sigma + 0.5);
+        if (G.r > MET_GMAX || !(sigma > 0)) { tmp.free_all(); return fail(HB2_ERR_GEOMETRY, "2-D metrics: unexpected rescale filter"); }
+        double sum = 0.0, wk[2 * MET_GMAX + 1];
+        for (int k = -G.r; k <= G.r; ++k) { wk[k + G.r] = std::exp(-0.5 / (sigma * sigma) * (double)(k * k)); }
+        for (int k = 0; k < 2 * G.r + 1; ++k) sum += wk[k];
+        for (int k = 0; k <= G.r; ++k) G.w[k] = wk[G.r + k] / sum;
+      }
+      const unsigned gb = cdiv((long long)H * W, HB2_BLOCK);
+      k_met_gauss<0><<<dim3(gb, nc + 1), HB2_BLOCK, 0, st>>>(im, stride, ta, HW, H, W, gy, nc, ms);
+      k_met_gauss<1><<<dim3(gb, nc + 1), HB2_BLOCK, 0, st>>>(ta, HW, tb, HW, H, W, gx, nc, ms);
+      k_met_zoom<<<dim3(cdiv((long long)Ho * Wo, HB2_BLOCK), nc + 1), HB2_BLOCK, 0, st>>>(
+          tb, HW, H, W, img + off[s + 1], stride, Ho, Wo, (double)H / Ho, (double)W / Wo, nc, ms, rng);
+      k_met_range<<<nc + 1, HB2_BLOCK, 0, st>>>(img + off[s + 1], stride, Ho * Wo, nc, ms, rng);
+      k_met_check<<<cdiv(nc, 128), 128, 0, st>>>(ms, rng, nc);
+    }
+  }
+  k_met_final<<<cdiv(nc, 128), 128, 0, st>>>(ms, nc, metric, b->d_cos, b->d_score, parts);
+  CKS(cudaGetLastError());
+  CKS(cudaEventRecord(e1, st));
+  if (scores_host) CKS(cudaMemcpyAsync(scores_host, b->d_score, sizeof(float) * nc, cudaMemcpyDeviceToHost, st));
+  if (all) CKS(cudaMemcpyAsync(parts_host, parts, sizeof(double) * 4 * nc, cudaMemcpyDeviceToHost, st));
+  CKS(cudaStreamSynchronize(st));
+  tmp.free_all();
+#undef CKS
+  float ms_m = 0;
+  cudaEventElapsedTime(&ms_m, e0, e1);
+  cudaEventDestroy(e0); cudaEventDestroy(e1);
+  b->timing[15] = ms_m;
   return HB2_OK;
 }
 

@@ -80,6 +80,9 @@ def main(argv=None):
                     help="solver model (app.py algorithm; default lsq)")
     ap.add_argument("--alpha", type=float, default=None, help="model alpha (default: 1 for ridge, 1e-4 otherwise)")
     ap.add_argument("--l1-ratio", type=float, default=None, help="elastic-net l1_ratio (default 0.5)")
+    ap.add_argument("--score-metric", default="cosine",
+                    choices=["cosine", "ssim", "ms_ssim", "mutual_information", "composite"],
+                    help="score that ranks the candidates (app.py score_metric; default cosine)")
     args = ap.parse_args(argv)
     algorithm = None
     if args.model != "lsq":
@@ -125,7 +128,8 @@ def main(argv=None):
                           positive_constraint=args.positive_constraint, top_k=args.top_k, device=local_rank,
                           shard=(rank, world), return_x_top=args.save_map, interpolation=args.interpolation, dist=dist,
                           checkpoint=f"{args.output}_img{i}.tiles" if args.resume else None,
-                          batch_candidates=args.batch_candidates or None, algorithm=algorithm)
+                          batch_candidates=args.batch_candidates or None, algorithm=algorithm,
+                          score_metric=args.score_metric)
         # with more than one process the per-rank score maps were all-gathered inside search_grid (one NCCL call)
         if rank != 0:
             continue
@@ -134,7 +138,7 @@ def main(argv=None):
                             rises=rises, csyms=np.array(csyms))
         top = [dict(score=e["score"], twist=e["twist"], rise=e["rise"], csym=e["csym"]) for e in out["top"]]
         report.append(dict(image=i, n_candidates=int(np.isfinite(out["scores"]).sum()), seconds=out["seconds"], top=top,
-                           n_restored=int(out.get("n_restored", 0))))
+                           n_restored=int(out.get("n_restored", 0)), score_metric=args.score_metric))
         best = out["top"][0] if out["top"] else None
         if best is not None:
             print(f"image {i}: best twist={best['twist']:.4f} rise={best['rise']:.4f} csym={best['csym']} "

@@ -267,6 +267,45 @@ class Batch:
         _lib.check(_lib.load().hb2_batch_model_info(self._h, int(c), _lib.ptr(out)))
         return dict(alpha=float(out[0]), iterations=int(out[1]), gap=float(out[2]), lipschitz=float(out[3]))
 
+    def pixel_rows(self, c):
+        """Last-writer table of candidate ``c`` over the (L2, D2) image: for pixel id k*D2 + j the padded data row that
+        _metric_2d's ``pred_2d.ravel()[pid] = pred`` leaves there (the last row of that pixel in the reference's order
+        (copy, k, j); numpy's fancy assignment keeps the last of repeated indices), or -1."""
+        pidx, kk, jj = self.data_row_index(c)
+        D2 = self.problem.D2
+        table = np.full(self.problem.L2 * D2, -1, dtype=np.int32)
+        table[(kk * D2 + jj).astype(np.int64)] = pidx
+        return table
+
+    def set_pixel_rows(self):
+        """Upload every candidate's pixel_rows table (hb2_batch_set_pixel_rows); the grid search does it on the
+        pipeline's worker thread while the previous batch is being solved."""
+        lib = _lib.load()
+        for c in range(self.nc):
+            t = self.pixel_rows(c)
+            _lib.check(lib.hb2_batch_set_pixel_rows(self._h, c, _lib.ptr(t), self.problem.L2, self.problem.D2))
+        self._pixel_rows_set = True
+
+    def score_metric(self, metric, clip_pred=0, parts=False):
+        """Replace every candidate's score by the 2-D ``metric`` ("ssim", "ms_ssim", "mutual_information",
+        "composite") of _metric_2d, computed on the device (hb2_batch_score_metric) after ``solve`` or ``solve_model``.
+        Returns the result array of that solve with the new scores; ``parts=True`` also returns [nc, 4] float64
+        (cosine, ssim, ms_ssim, mutual information)."""
+        if metric not in _lib.METRICS:
+            raise ValueError(f"unknown score_metric {metric!r}")
+        if self.results is None:
+            raise _lib.HeliconB200Error("Batch.score_metric before a solve")
+        if not getattr(self, "_pixel_rows_set", False):
+            self.set_pixel_rows()
+        sc = np.empty(self.nc, dtype=np.float32)
+        out = np.empty((self.nc, 4), dtype=np.float64) if parts else None
+        _lib.check(_lib.load().hb2_batch_score_metric(self._h, _lib.METRICS[metric], int(clip_pred), _lib.ptr(sc),
+                                                      _lib.ptr(out) if parts else None))
+        res = self.results.copy()
+        res["score"] = sc
+        self.results = res
+        return (res, out) if parts else res
+
     def apply_all(self, xs=None, ys=None):
         """The MODE_PLAIN products over all candidates in one launch each (tests): ``xs`` [nc, n] -> list of row
         vectors, or ``ys`` (list of row vectors) -> [nc, n]."""
@@ -288,7 +327,8 @@ class Batch:
         _lib.check(_lib.load().hb2_batch_timing(self._h, _lib.ptr(out)))
         return dict(lsmr_ms=out[0], trf_ms=out[1], score_ms=out[2], launches=int(out[3]), iterations=int(out[4]),
                     fwd_data_ms=out[5], fwd_sym_ms=out[6], adj_ms=out[7], update_ms=out[8], scalar_ms=out[9],
-                    fwd_data_launches=int(out[10]), adj_launches=int(out[11]), update_launches=int(out[12]), norm_ms=out[14])
+                    fwd_data_launches=int(out[10]), adj_launches=int(out[11]), update_launches=int(out[12]), norm_ms=out[14],
+                    metric_ms=out[15])
 
     def trf_trace(self, c):
         out = np.zeros((24, 8), dtype=np.float64)

@@ -303,7 +303,8 @@ def search_grid(image, apix, twists, rises, csyms=(1,), reconstruct_length_rise=
                 tube_diameter_inner=0.0, tube_length=None, target_apix3d=0, sym_oversample=-1,
                 positive_constraint=-1, thresh_fraction=-1, top_k=10, device=0, stream=None, batch_candidates=None,
                 mem_budget_bytes=48 << 30, shard=(0, 1), return_x_top=False, progress=None, pipelined=True,
-                interpolation="nn", dist=None, checkpoint=None, checkpoint_seconds=30.0, algorithm=None):
+                interpolation="nn", dist=None, checkpoint=None, checkpoint_seconds=30.0, algorithm=None,
+                score_metric="cosine"):
     """Solve + score every candidate of the grid on one GPU (or this rank's share of it).
 
     ``interpolation="nn"`` runs batches of candidates through the matrix-free projector; ``"linear"`` (trilinear rows,
@@ -325,10 +326,15 @@ def search_grid(image, apix, twists, rises, csyms=(1,), reconstruct_length_rise=
     ``{"model": "elasticnet" | "lasso" | "ridge", "alpha": .., "l1_ratio": ..}`` the batched model solver
     (Batch.solve_model) with the reference's defaults; other models and ``interpolation="linear"`` with a model raise
     NotImplementedError before any GPU work.
+    ``score_metric`` (SLR:484-525): "cosine" (default, the solve's own score) or "ssim" / "ms_ssim" /
+    "mutual_information" / "composite", computed for every candidate on the device after its batch's solve
+    (Batch.score_metric) with the semantics of ``lsq_reconstruct(..., score_metric=...)``; the score map, top-K,
+    checkpoint tiles and ``return_x_top`` then rank by it.
     Returns dict(scores[(n_csym,) T, R] (NaN = not solved here / skipped task), itn, flags, top,
     n_candidates, seconds).
     """
     mparams = check_algorithm(algorithm, interpolation)
+    check_score_metric(score_metric)
     ny, nx = np.asarray(image).shape
     tube_d = ny * apix if tube_diameter is None else tube_diameter
     image = prepare_image(image, thresh_fraction, tube_d if 0 < tube_d < ny * apix else ny * apix, apix)
@@ -350,7 +356,7 @@ def search_grid(image, apix, twists, rises, csyms=(1,), reconstruct_length_rise=
                          tube_diameter_inner=tube_diameter_inner, tube_length=tube_length, target_apix3d=target_apix3d,
                          sym_oversample=sym_oversample, positive_constraint=positive_constraint,
                          clip_pred=int(thresh_fraction >= 0), interpolation=str(interpolation), library=_version(),
-                         **model_fingerprint(mparams))
+                         **model_fingerprint(mparams), **metric_fingerprint(score_metric))
         store = ScoreTileStore(checkpoint, fp, ntot, rank=rank, world=world, flush_seconds=checkpoint_seconds)
         if world > 1 and dist is not None and dist.is_available() and dist.is_initialized():
             agree_across_ranks(store, dist, device)  # every rank must filter the SAME tasks
@@ -391,7 +397,8 @@ def search_grid(image, apix, twists, rises, csyms=(1,), reconstruct_length_rise=
 
     try:
         stats = solve_chunks(chunks, queue, problem, device=device, pipelined=pipelined, interpolation=interpolation,
-                             clip_pred=int(thresh_fraction >= 0), on_result=on_result, algorithm=algorithm if mparams else None)
+                             clip_pred=int(thresh_fraction >= 0), on_result=on_result, algorithm=algorithm if mparams else None,
+                             score_metric=score_metric)
         n_solved = stats["n_candidates"]
         if dist is not None and dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
             # the ONLY collective of a search: every rank's maps all-gathered (NCCL), folded and ranked on the device
@@ -434,7 +441,7 @@ def search_grid(image, apix, twists, rises, csyms=(1,), reconstruct_length_rise=
 
 
 TIMING_KEYS = ("lsmr_ms", "trf_ms", "score_ms", "fwd_data_ms", "fwd_sym_ms", "adj_ms", "update_ms", "scalar_ms", "norm_ms",
-               "launches", "fwd_data_launches", "adj_launches", "update_launches")
+               "metric_ms", "launches", "fwd_data_launches", "adj_launches", "update_launches")
 
 
 def model_fingerprint(mparams):
@@ -445,14 +452,27 @@ def model_fingerprint(mparams):
     return dict(model=model, alpha=float(alpha), l1_ratio=float(l1_ratio))
 
 
+def check_score_metric(score_metric):
+    """The score metrics lsq_reconstruct accepts; raises before any GPU work."""
+    if score_metric not in ("cosine", "ssim", "ms_ssim", "mutual_information", "composite"):
+        raise ValueError(f"unknown score_metric {score_metric!r}")
+
+
+def metric_fingerprint(score_metric):
+    """Checkpoint parameter of the score metric: none for cosine, so that the tiles of existing searches resume."""
+    return {} if score_metric == "cosine" else dict(score_metric=str(score_metric))
+
+
 def solve_chunks(chunks, queue, problem_of, device=0, pipelined=True, interpolation="nn", clip_pred=0, profile=0,
-                 on_result=None, solve_options=None, algorithm=None):
+                 on_result=None, solve_options=None, algorithm=None, score_metric="cosine"):
     """Solve the chunks ``queue`` deals to this rank: ``chunks[i] = (problem key, [GridTask], cost)`` (make_chunks).
 
     The batch of chunk i+1 is planned and set up by a worker thread (second stream) while chunk i is being solved
     (BatchPipeline).  ``on_result(chunk_tasks, results, batch)`` is called per solved batch, before it is closed.
     Returns the summed library timings (``profile=1`` adds the per-kernel-class device times).  ``algorithm``: a
-    sklearn-model dict solves every batch with Batch.solve_model instead of LSMR."""
+    sklearn-model dict solves every batch with Batch.solve_model instead of LSMR.  ``score_metric`` other than "cosine":
+    every batch is re-scored with Batch.score_metric after its solve; its pixel tables are built with the batch on the
+    worker thread."""
     pipe = BatchPipeline(device=device, pipelined=pipelined)
     stats = dict.fromkeys(TIMING_KEYS, 0.0)
     stats.update(n_candidates=0, n_chunks=0, itn_sum=0, chunk_ids=[])
@@ -470,6 +490,18 @@ def solve_chunks(chunks, queue, problem_of, device=0, pipelined=True, interpolat
                     raise AssertionError("explicit rows: one candidate per batch")
                 return ExplicitBatch(prob, L3, specs[0], interpolation=interpolation, stream=stream)
 
+        if score_metric != "cosine":
+            build = factory or (lambda prob, L3, specs, stream: Batch(prob, L3, specs, stream=stream))
+
+            def factory(prob, L3, specs, stream):
+                batch = build(prob, L3, specs, stream)
+                try:
+                    batch.set_pixel_rows()
+                except BaseException:
+                    batch.close()
+                    raise
+                return batch
+
         batches = pipe.run_items(((problem_of(chunks[ci][0]), chunks[ci][0][5], [x.spec for x in chunks[ci][1]], ci)
                                   for ci in queue), factory)
         for ci, batch in batches:
@@ -479,6 +511,8 @@ def solve_chunks(chunks, queue, problem_of, device=0, pipelined=True, interpolat
                     res = batch.solve_model(algorithm, clip_pred=clip_pred, **opts)
                 else:
                     res = batch.solve(clip_pred=clip_pred, profile=int(profile), **opts)
+                if score_metric != "cosine":
+                    res = batch.score_metric(score_metric, clip_pred=clip_pred)
                 tm = batch.timing()
                 for k in TIMING_KEYS:
                     stats[k] += tm.get(k, 0.0)
@@ -494,7 +528,7 @@ def solve_chunks(chunks, queue, problem_of, device=0, pipelined=True, interpolat
         if batches is not None and hasattr(batches, "close"):
             batches.close()  # closes a batch the worker thread may still be building, BEFORE the problems go away
         pipe.close()
-    stats["kernel_ms"] = stats["lsmr_ms"] + stats["trf_ms"] + stats["score_ms"]
+    stats["kernel_ms"] = stats["lsmr_ms"] + stats["trf_ms"] + stats["score_ms"] + stats["metric_ms"]
     stats["launches"] = int(stats["launches"])
     return stats
 

@@ -1,6 +1,8 @@
 """Host-side image preparation and 2-D score metrics of the denovo3D task wrapper (SURVEY.md section 8f ranks 3-4).
 
-These run once per TASK on one small 2-D image (not per voxel or per iteration) and are outside the CUDA hot path; the
+``process_one_task`` / ``lsq_reconstruct`` run these once per TASK on one small 2-D image, on the host.  A grid search
+scores every candidate, so ``search_grid(score_metric=...)`` runs the same three metrics on the device instead
+(csrc/hb2_metric.cuh, Batch.score_metric), following these functions exactly.  The
 reference implements them with scikit-image, which exists neither in the build container nor on the GPU box, so the
 functions below RESTATE the published algorithms of the scikit-image 0.2x calls the reference makes with numpy /
 scipy.ndimage.  **Parity unpinned**: the reference's own calls cannot be executed here (ImportError), so no golden

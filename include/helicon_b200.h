@@ -303,7 +303,8 @@ int hb2_batch_get_x(hb2_batch* b, int32_t cand, float* x_host);
  * [0] lsmr phase ms, [1] trf phase ms, [2] score phase ms, [3] kernels launched, [4] lsmr iterations run,
  * with opt.profile=1 also per kernel class, summed over launches (ms) and launch counts:
  * [5] fwd_data ms [6] fwd_sym ms [7] adjoint ms [8] update ms [9] scalar kernels ms,
- * [10] fwd_data launches [11] adjoint launches [12] update launches, [13..15] reserved */
+ * [10] fwd_data launches [11] adjoint launches [12] update launches, [13..14] reserved,
+ * [15] device ms of the last hb2_batch_score_metric (0 before one) */
 int hb2_batch_timing(hb2_batch* b, double* out16);
 
 /* debug/test: per outer iteration of the bounded branch of the last solve, out[row*8 + k] =
@@ -345,6 +346,25 @@ int hb2_batch_model_info(hb2_batch* b, int32_t cand, double* out4);
  * ([nc][n], reference order), out = rows ([nc][total padded rows of hb2_batch_rows_padded] concatenated); adjoint = 1:
  * the other way round. */
 int hb2_batch_apply_all(hb2_batch* b, int32_t adjoint, const float* in_host, float* out_host);
+
+/* ---- 2-D score metrics (SLR:484-525, helicon_b200/imageprep.py) for every candidate of a solved batch -----------
+ * The candidate's prediction A_data x (float32 x of hb2_batch_get_x, MODE_PLAIN forward, clipped at 0 when clip_pred)
+ * is scattered into pred_2d[L2][D2] and scored against the transposed central (D2, L2) region of the problem's image
+ * (the image hb2_problem_create received).  The metric's value replaces the candidate's score (the buffer that
+ * hb2_batch_scatter_scores reads); composite is the mean of [cosine, ssim, ms_ssim, mutual information], its cosine
+ * part the score the solve computed. */
+#define HB2_METRIC_SSIM 1
+#define HB2_METRIC_MS_SSIM 2
+#define HB2_METRIC_MI 3
+#define HB2_METRIC_COMPOSITE 4
+/* The candidate's pixel table: last_row[k*D2 + j] = the padded data row (Batch.data_row_index) that writes pixel
+ * (k, j) last in the reference's row order (copy, k, j), or -1 where no row does.  Every entry must be < the candidate's
+ * padded data rows.  Required for every candidate before hb2_batch_score_metric. */
+int hb2_batch_set_pixel_rows(hb2_batch* b, int32_t cand, const int32_t* last_row, int32_t L2, int32_t D2);
+/* After hb2_batch_solve / hb2_batch_solve_model (HB2_ERR_STATE otherwise, or without the pixel tables).  scores_host
+ * [nc] (nullable): the new scores; parts_host [nc][4] (nullable): cosine, ssim, ms_ssim, mutual information in
+ * float64.  The device time of the call is hb2_batch_timing's out[15]. */
+int hb2_batch_score_metric(hb2_batch* b, int32_t metric, int32_t clip_pred, float* scores_host, double* parts_host);
 
 /* ---- test hook: the LSMR scalar recurrences run on the HOST --------------- */
 /* Same code as the device path (compiled __host__ __device__).  state64 is an
